@@ -21,6 +21,9 @@ contiguous slab of its slices; the engine all-gathers the argmax slabs itself (C
 and every rank post-processes the whole volume -> strong scaling of one volume's latency.
 The line also carries the parity of the run: Dice / argmax flips / differing voxels of the engine against the CPU
 oracle on the bounded sample the CPU baseline is timed on.
+--dump-outputs DIR writes what the timed path returned in its last timed step (rank 0's label volumes) as
+DIR/<name>.npy in float32, so that two builds run with the same arguments (same seeded volumes and weights) can be
+compared output for output.
 """
 import argparse
 import json
@@ -55,10 +58,25 @@ WEIGHT_SEEDS = {3: 7, 6: 8}
 # mean dram__bytes_read.sum + dram__bytes_write.sum per conv_tc_kernel launch: taken from the newest committed ncu --set full
 # summary that tools/ncu_summarize.py wrote (profiles/*conv_traffic.json: per-layer table of one full 37-slice wave)
 TRAFFIC_FALLBACK = (188.7e6, "profiles/r01_ncu_summary_v5.md (4 launches of a 37-slice wave, layers down2/down3)")
+DUMP_BYTES = 64 * 10**6   # --dump-outputs writes at most this much in all
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes every {name: array} as out_dir/<name>.npy in float32.  An output larger than its share of DUMP_BYTES is
+    written as a fixed sample instead: its values at seeded random flat indices, in index order, as a 1-D array."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = (DUMP_BYTES // len(outputs) - 4096) // 4   # float32 elements per file, room left for the .npy header
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        if a.size > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))
+            log("dump %s: %d of %d values of shape %s (seeded sample)" % (name, share, a.size, a.shape))
+            a = a.ravel()[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def rank_info():
@@ -168,8 +186,10 @@ def run_reference(args):
         cpu_port(cfg, sds, sample)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_port(cfg, sds, sample)
+        _, out = cpu_port(cfg, sds, sample)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"labels": out})
     v = n * args.steps / dt
     cores = torch.get_num_threads()
     line = {"impl": "reference", "metric": "CT slices/sec @256x256 (%s)" % ("R231" if args.config in ("C2", "C5") else args.config), "value": v, "unit": "slices/s", "n_gpus": args.gpus,
@@ -268,6 +288,7 @@ def run_engine(args):
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
     sampler.stop_flag = True
+    last_step = {"labels_vol%d" % i: d.cpu().numpy() for i, d in enumerate(d_outs)} if (args.dump_outputs and rank == 0) else None
     # every engine call ends with a stream synchronisation, so the bracketed wall time between the two synchronised
     # barriers IS the device-side duration of the K steps
     step_ms = wall_ms / args.steps
@@ -369,6 +390,8 @@ def run_engine(args):
                              "sample": "first %d slices of the same volume, full path (oracle port of mask.py:141-232)" % n_cpu},
         }
         print(json.dumps(line), flush=True)
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, last_step)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -382,7 +405,10 @@ def main():
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--config", default="C2", choices=sorted(CONFIGS))
     ap.add_argument("--mode", default="replica", choices=["replica", "shard"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

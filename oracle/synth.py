@@ -140,7 +140,18 @@ def random_state_dict(K: int, seed: int, calibrate_on: np.ndarray = None, head_g
     return sd
 
 
-def _forward_train(x, sd, momentum):
+def _upsample2x(x):
+    """F.interpolate(x, scale_factor=2, mode="bilinear", align_corners=False) from slices and sums, whose backward
+    is deterministic on CUDA (F.interpolate's accumulates with atomics)."""
+    for d in (2, 3):
+        n = x.shape[d]
+        prev = torch.cat([x.narrow(d, 0, 1), x.narrow(d, 0, n - 1)], d)
+        nxt = torch.cat([x.narrow(d, 1, n - 1), x.narrow(d, n - 1, 1)], d)
+        x = torch.stack([0.25 * prev + 0.75 * x, 0.75 * x + 0.25 * nxt], d + 1).flatten(d, d + 1)
+    return x
+
+
+def _forward_train(x, sd, momentum, upsample=None):
     """Same graph as restate.unet_forward but with BN in training mode (updates running stats)."""
     def block(x, p):
         for conv, bn in ((0, 2), (3, 5)):
@@ -156,7 +167,7 @@ def _forward_train(x, sd, momentum):
             skips.append(x)
             x = F.avg_pool2d(x, 2)
     for j in range(4):
-        up = F.interpolate(x, scale_factor=2, mode="bilinear", align_corners=False)
+        up = upsample(x) if upsample else F.interpolate(x, scale_factor=2, mode="bilinear", align_corners=False)
         up = F.conv2d(up, sd[f"up_path.{j}.up.1.weight"], sd[f"up_path.{j}.up.1.bias"])
         x = block(torch.cat([up, skips[-j - 1]], 1), f"up_path.{j}.conv_block.block")
     return F.log_softmax(F.conv2d(x, sd["last.weight"], sd["last.bias"]), dim=1)
@@ -175,7 +186,8 @@ def train_state_dict(K: int, seed: int, steps: int = 60, device: str = None, n_s
                      batch: int = 4, lr: float = 1e-3, log=None) -> OrderedDict:
     """'Trained-looking' weights: a few Adam steps on phantom ground truth so the label maps are
     clean blobs (~2 components per slice) instead of speckle (SURVEY.md Appendix A).  Harness-only
-    use of torch autograd; runs on cuda when available (seconds) else CPU (minutes)."""
+    use of torch autograd; runs on cuda when available (seconds) else CPU (minutes).  The steps use
+    only deterministic kernels, so the same arguments give the same weights on every run."""
     if device is None:
         device = "cuda" if torch.cuda.is_available() else "cpu"
     g = torch.Generator().manual_seed(seed)
@@ -189,14 +201,20 @@ def train_state_dict(K: int, seed: int, steps: int = 60, device: str = None, n_s
     for k in params:
         sd[k].requires_grad_(True)
     opt = torch.optim.Adam([sd[k] for k in params], lr=lr)
-    for step in range(steps):
-        idx = torch.randint(0, n_slices, (batch,), generator=g).to(device)
-        loss = F.nll_loss(_forward_train(x_all[idx], sd, momentum=0.1), y_all[idx])
-        opt.zero_grad(set_to_none=True)
-        loss.backward()
-        opt.step()
-        if log is not None and (step % 10 == 0 or step == steps - 1):
-            log(f"train K={K} step {step} loss {loss.item():.4f}")
+    cudnn_deterministic = torch.backends.cudnn.deterministic
+    torch.backends.cudnn.deterministic = True
+    try:
+        for step in range(steps):
+            idx = torch.randint(0, n_slices, (batch,), generator=g).to(device)
+            logp = _forward_train(x_all[idx], sd, momentum=0.1, upsample=_upsample2x)
+            loss = -(logp * F.one_hot(y_all[idx], K).permute(0, 3, 1, 2)).sum(1).mean()   # F.nll_loss without atomics
+            opt.zero_grad(set_to_none=True)
+            loss.backward()
+            opt.step()
+            if log is not None and (step % 10 == 0 or step == steps - 1):
+                log(f"train K={K} step {step} loss {loss.item():.4f}")
+    finally:
+        torch.backends.cudnn.deterministic = cudnn_deterministic
     for k in params:
         sd[k].requires_grad_(False)
     with torch.no_grad():  # re-calibrate BN on a fixed batch, in eval-compatible form

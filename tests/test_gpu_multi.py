@@ -53,7 +53,7 @@ def _worker(rank, world, port, q):
 def test_sharded_volume_equals_single_gpu():
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     import torch.multiprocessing as mp
     world = int(os.environ.get("LM_TEST_WORLD", min(torch.cuda.device_count(), 4)))   # 2 ranks, or 4 on a box with >= 4 GPUs
     ctx = mp.get_context("spawn")
