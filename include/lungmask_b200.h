@@ -131,6 +131,31 @@ LM_API int lm_apply_volume_sharded(lm_engine* e, int slot, const int16_t* vol, i
 LM_API int lm_apply_volume_sharded_dev(lm_engine* e, int slot, const int16_t* d_vol, int S, int H, int W, int flags,
                                        uint8_t* d_out);
 
+/* ---- compressed DICOM pixel data (what SimpleITK / GDCM decode for utils.read_dicoms, utils.py:186-190) -----------
+ * lm_decode_frames decodes n_frames single-component 16-bit frames, each encoded in data[offset, offset + length):
+ *   LM_CODEC_JPEG_LOSSLESS  ITU-T T.81 process 14 (SOF3, Huffman): predictors 1-7, point transform, restart intervals
+ *                           of whole rows; transfer syntaxes 1.2.840.10008.1.2.4.57 and .4.70
+ *   LM_CODEC_RLE            DICOM PS3.5 Annex G (1.2.840.10008.1.2.5): exactly 2 segments, most significant bytes first
+ * into out as stored 16-bit values, the frames one after the other (frame i starts at the sum of rows * cols of the
+ * frames before it).  With is_signed and a JPEG precision P < 16 the values are sign-extended from bit P - 1.
+ * frame_status[i] is 0 or one of LM_ERR_DECODE_* (a failed frame's output is unspecified).  The call returns 0 once
+ * every frame has a status, non-zero (lm_last_error) for invalid arguments or a CUDA error.  It needs no engine: it
+ * runs on `device` with its own stream and scratch memory, frees both and synchronises before it returns.  All
+ * pointers are host pointers. */
+#define LM_CODEC_JPEG_LOSSLESS 1
+#define LM_CODEC_RLE 2
+#define LM_ERR_DECODE_HEADER (-60) /* unsupported or malformed JPEG marker segments (frame type, Nf, size, EOI) or RLE header */
+#define LM_ERR_DECODE_DATA (-61)   /* entropy-coded data: undefined Huffman code, unexpected marker, RSTm out of sequence */
+#define LM_ERR_DECODE_LENGTH (-62) /* JPEG: a restart interval ends before its samples, or the RSTm count differs from the
+                                      * number of intervals (codewords after the last sample are ignored, as libjpeg-turbo
+                                      * does); RLE: a segment ends before, or runs past, rows * cols bytes */
+typedef struct {
+  uint64_t offset, length;
+  int32_t codec, rows, cols, is_signed;
+} lm_frame;
+LM_API int lm_decode_frames(int device, const uint8_t* data, size_t n_bytes, const lm_frame* frames, int n_frames,
+                            uint16_t* out, int32_t* frame_status);
+
 /* ---- stage-level entry points (each mirrors one reference function; used by the parity tests) ---- */
 
 /* utils.preprocess(img, resolution=[out_h,out_w]), utils.py:32-52 (+ simple_bodymask :55-82,

@@ -63,6 +63,7 @@ def lib():
         "lm_debug_activation_info": ([i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)], i32),
         "lm_debug_read_activation": ([vp, i32, i32, f32p], i32),
         "lm_last_conv_timing": ([vp, C.POINTER(C.c_float), C.POINTER(C.c_int64)], i32),
+        "lm_decode_frames": ([i32, u8p, C.c_size_t, vp, i32, vp, i32p], i32),
     }
     for name, (argtypes, restype) in sig.items():
         fn = getattr(L, name)  # AttributeError here = header / library mismatch
@@ -78,7 +79,28 @@ EXPORTS = ["lm_create", "lm_destroy", "lm_last_error", "lm_device", "lm_batch_ca
            "lm_simple_bodymask", "lm_forward", "lm_forward_dev", "lm_postprocess", "lm_reshape_masks",
            "lm_keep_largest_component",
            "lm_last_timings", "lm_set_option", "lm_last_conv_timing",
-           "lm_debug_activation_info", "lm_debug_read_activation"]
+           "lm_debug_activation_info", "lm_debug_read_activation", "lm_decode_frames"]
+
+
+CODEC_JPEG_LOSSLESS, CODEC_RLE = 1, 2
+DECODE_ERRORS = {-60: "unsupported or malformed JPEG marker segments or RLE header",
+                 -61: "malformed entropy-coded data",
+                 -62: "the data ends before Rows x Columns samples or does not match the restart intervals"}
+FRAME_DTYPE = np.dtype([("offset", "<u8"), ("length", "<u8"), ("codec", "<i4"), ("rows", "<i4"), ("cols", "<i4"),
+                        ("is_signed", "<i4")])   # lm_frame
+
+
+def decode_frames(data, frames, device=0):
+    """lm_decode_frames: `data` bytes, `frames` a FRAME_DTYPE array -> (list of (rows, cols) uint16 arrays, int32 status
+    per frame).  Needs no Engine."""
+    frames = np.ascontiguousarray(frames, dtype=FRAME_DTYPE)
+    buf = np.frombuffer(data, dtype=np.uint8) if len(data) else np.zeros(1, np.uint8)
+    sizes = frames["rows"].astype(np.int64) * frames["cols"].astype(np.int64)
+    out = np.empty(int(sizes.sum()), np.uint16)
+    status = np.zeros(len(frames), np.int32)
+    _check(lib().lm_decode_frames(int(device), _ptr(buf), len(data), _ptr(frames), len(frames), _ptr(out), _ptr(status)))
+    ends = np.cumsum(sizes)
+    return [out[e - n:e].reshape(int(r), int(c)) for e, n, r, c in zip(ends, sizes, frames["rows"], frames["cols"])], status
 
 
 def _ptr(a):

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "liblungmask_b200.so")
-SOURCES = ["conv_tc.cu", "conv_tc_pair.cu", "forward_misc.cu", "preproc.cu", "postproc.cu", "shard.cu", "engine.cu"]
+SOURCES = ["conv_tc.cu", "conv_tc_pair.cu", "forward_misc.cu", "preproc.cu", "postproc.cu", "shard.cu", "engine.cu", "decode.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

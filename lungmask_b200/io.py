@@ -5,8 +5,9 @@ The reference leans on SimpleITK (ITK / GDCM) and pydicom for this; neither is i
 only needs three things from a file: the voxel array (z, y, x), the 3x3 direction cosines (for the orientation
 handling of mask.py:157-164) and enough geometry to write the mask back next to the input.  So this module reads
 
-  * DICOM series (a directory tree): uncompressed little-endian transfer syntaxes (implicit / explicit VR), 16-bit
-    pixels, RescaleSlope / RescaleIntercept applied as ITK does; slices grouped by SeriesInstanceUID, de-duplicated by
+  * DICOM series (a directory tree): uncompressed little-endian transfer syntaxes (implicit / explicit VR), and JPEG
+    Lossless (.4.57, .4.70) and RLE Lossless (.5) single-frame encapsulated pixel data, decoded on the GPU by
+    lm_decode_frames in one call per series; 16-bit pixels, RescaleSlope / RescaleIntercept applied as ITK does; slices grouped by SeriesInstanceUID, de-duplicated by
     (study, series, position) and sorted by the z component of ImagePositionPatient exactly like utils.py:196-214;
     the largest series wins (utils.py:262-268); ImageType filters `primary` / `original` as in utils.py:152-170;
   * NIfTI-1 single files (.nii, .nii.gz): sform, else qform, else pixdim; RAS -> LPS like ITK's NIfTI reader;
@@ -46,11 +47,12 @@ class Volume:
 # --------------------------------------------------------------------------------------------------------------
 _LONG_VR = {b"OB", b"OW", b"OF", b"SQ", b"UT", b"UN", b"OD", b"OL", b"UC", b"UR", b"OV", b"SV", b"UV"}
 _EXPLICIT_LE, _IMPLICIT_LE = "1.2.840.10008.1.2.1", "1.2.840.10008.1.2"
+_CODECS = {"1.2.840.10008.1.2.4.57": 1, "1.2.840.10008.1.2.4.70": 1, "1.2.840.10008.1.2.5": 2}   # lm_frame.codec
 _WANTED = {(0x0008, 0x0008): "ImageType", (0x0020, 0x000D): "StudyInstanceUID", (0x0020, 0x000E): "SeriesInstanceUID",
            (0x0020, 0x0032): "ImagePositionPatient", (0x0020, 0x0037): "ImageOrientationPatient", (0x0028, 0x0010): "Rows",
            (0x0028, 0x0011): "Columns", (0x0028, 0x0030): "PixelSpacing", (0x0028, 0x0100): "BitsAllocated",
            (0x0028, 0x0103): "PixelRepresentation", (0x0028, 0x1052): "RescaleIntercept", (0x0028, 0x1053): "RescaleSlope",
-           (0x0028, 0x0002): "SamplesPerPixel", (0x0018, 0x0050): "SliceThickness"}
+           (0x0028, 0x0002): "SamplesPerPixel", (0x0018, 0x0050): "SliceThickness", (0x0028, 0x0008): "NumberOfFrames"}
 
 
 class DicomError(ValueError):
@@ -84,7 +86,29 @@ def _skip_items(b, pos, explicit):
     return pos
 
 
-def _read_element(b, pos, explicit, want_value=True):
+def _read_fragments(b, pos):
+    """Encapsulated pixel data (PS3.5 A.4) from the first item on: Basic Offset Table item, fragment items, sequence
+    delimiter -> (fragment spans, position after the delimiter)."""
+    items = []
+    while True:
+        if pos + 8 > len(b):
+            raise DicomError("encapsulated pixel data without a sequence delimiter")
+        g, e, ln = struct.unpack_from("<HHI", b, pos)
+        pos += 8
+        if (g, e) == (0xFFFE, 0xE0DD):
+            break
+        if (g, e) != (0xFFFE, 0xE000) or ln == 0xFFFFFFFF or pos + ln > len(b):
+            raise DicomError("malformed encapsulated pixel data")
+        items.append((pos, ln))
+        pos += ln
+    if len(items) < 2:
+        raise DicomError("encapsulated pixel data without a fragment")
+    if items[0][1] > 4:
+        raise DicomError("multi-frame objects are not supported")
+    return items[1:], pos
+
+
+def _read_element(b, pos, explicit, want_value=True, encapsulated=False):
     g, e = struct.unpack_from("<HH", b, pos)
     if explicit and g != 0xFFFE:
         vr = b[pos + 4:pos + 6]
@@ -100,13 +124,16 @@ def _read_element(b, pos, explicit, want_value=True):
         vpos = pos + 8
     if ln == 0xFFFFFFFF:                    # undefined length: a sequence (or encapsulated pixel data)
         if (g, e) == (0x7FE0, 0x0010):
-            raise DicomError("encapsulated (compressed) pixel data is not supported")
+            if not encapsulated:
+                raise DicomError("encapsulated (compressed) pixel data is not supported")
+            frags, end = _read_fragments(b, vpos)
+            return end, (g, e), (frags if want_value else None)
         return _skip_sequence(b, vpos, explicit), (g, e), None
     return vpos + ln, (g, e), ((vpos, ln) if want_value else None)
 
 
-def read_dicom_file(path, stop_before_pixels=False):
-    """-> dict of the tags this module needs (+ 'pixels': int16/uint16 2-D array unless stop_before_pixels)."""
+def _read_dicom(path, stop_before_pixels=False):
+    """read_dicom_file without the decode: a compressed frame is left in '_frame' = (codec, bytes)."""
     with open(path, "rb") as f:
         b = f.read()
     pos, syntax = 0, _IMPLICIT_LE
@@ -118,15 +145,17 @@ def read_dicom_file(path, stop_before_pixels=False):
                 syntax = b[val[0]:val[0] + val[1]].decode("ascii", "ignore").strip("\x00 ")
     elif len(b) < 8:
         raise DicomError("not a DICOM file")
-    if syntax not in (_EXPLICIT_LE, _IMPLICIT_LE):
-        raise DicomError("transfer syntax %s is not supported (uncompressed little endian only)" % syntax)
-    explicit = syntax == _EXPLICIT_LE
+    codec = _CODECS.get(syntax)
+    if syntax not in (_EXPLICIT_LE, _IMPLICIT_LE) and codec is None:
+        raise DicomError("transfer syntax %s is not supported (uncompressed little endian, JPEG Lossless and RLE Lossless "
+                         "only)" % syntax)
+    explicit = syntax != _IMPLICIT_LE
     out = {}
     while pos + 8 <= len(b):
         g, e = struct.unpack_from("<HH", b, pos)
         if (g, e) == (0x7FE0, 0x0010) and stop_before_pixels:
             break
-        pos, tag, val = _read_element(b, pos, explicit)
+        pos, tag, val = _read_element(b, pos, explicit, encapsulated=codec is not None)
         if val is None:
             continue
         if tag in _WANTED:
@@ -144,6 +173,14 @@ def read_dicom_file(path, stop_before_pixels=False):
             raise DicomError("no pixel data")
         if out.get("BitsAllocated", 16) != 16 or out.get("SamplesPerPixel", 1) != 1:
             raise DicomError("only 16-bit single-sample images are supported")
+        if codec is not None:
+            if int(out.get("NumberOfFrames", "1") or 1) != 1:
+                raise DicomError("multi-frame objects are not supported")
+            span = out.pop("_pixel_span")
+            if not isinstance(span, list):              # a (vpos, length) tuple: native pixel data
+                raise DicomError("%s: transfer syntax %s requires encapsulated pixel data" % (path, syntax))
+            out["_frame"] = (codec, b"".join(b[p:p + n] for p, n in span))
+            return out
         vpos, ln = out.pop("_pixel_span")
         n = out["Rows"] * out["Columns"]
         if ln < 2 * n:
@@ -155,6 +192,43 @@ def read_dicom_file(path, stop_before_pixels=False):
     return out
 
 
+def _decode_device(device):
+    return int(os.environ.get("LOCAL_RANK", 0)) if device is None else int(device)
+
+
+def _decode_pending(slices, names, device=None):
+    """Decodes the compressed frames among `slices` (dicts of _read_dicom) in one lm_decode_frames call and stores each
+    as 'pixels' (int16 when PixelRepresentation is 1, else uint16, as for uncompressed data)."""
+    todo = [k for k, s in enumerate(slices) if "_frame" in s]
+    if not todo:
+        return
+    from . import _native
+    frames = np.zeros(len(todo), _native.FRAME_DTYPE)
+    blobs, off = [], 0
+    for i, k in enumerate(todo):
+        s = slices[k]
+        codec, blob = s["_frame"]
+        frames[i] = (off, len(blob), codec, s["Rows"], s["Columns"], 1 if s.get("PixelRepresentation", 0) == 1 else 0)
+        blobs.append(blob)
+        off += len(blob)
+    arrays, status = _native.decode_frames(b"".join(blobs), frames, _decode_device(device))
+    for i, k in enumerate(todo):
+        if status[i]:
+            raise DicomError("%s: cannot decode the compressed pixel data: %s (%d)"
+                             % (names[k], _native.DECODE_ERRORS.get(int(status[i]), "error"), int(status[i])))
+        s = slices[k]
+        del s["_frame"]
+        s["pixels"] = arrays[i].view(np.int16) if s.get("PixelRepresentation", 0) == 1 else arrays[i]
+
+
+def read_dicom_file(path, stop_before_pixels=False, device=None):
+    """-> dict of the tags this module needs (+ 'pixels': int16/uint16 2-D array unless stop_before_pixels).  Compressed
+    pixel data is decoded on CUDA device `device` (default: LOCAL_RANK, else 0)."""
+    out = _read_dicom(path, stop_before_pixels)
+    _decode_pending([out], [path], device)
+    return out
+
+
 def _floats(s, n):
     v = [float(x) for x in s.split("\\") if x.strip() != ""]
     if len(v) != n:
@@ -162,15 +236,16 @@ def _floats(s, n):
     return v
 
 
-def read_dicoms(path, primary=True, original=True, disable_tqdm=False, read_metadata=False):
-    """utils.read_dicoms (utils.py:132-232): every series under `path` as a Volume."""
+def read_dicoms(path, primary=True, original=True, disable_tqdm=False, read_metadata=False, device=None):
+    """utils.read_dicoms (utils.py:132-232): every series under `path` as a Volume.  The compressed frames of a series
+    are decoded in one call on CUDA device `device` (default: LOCAL_RANK, else 0)."""
     files = [os.path.join(d, f) for d, _, fs in os.walk(path) for f in fs]
     infos, seen = [], set()
     for fname in files:
         if os.path.splitext(os.path.basename(fname))[0] == "DICOMDIR":
             continue
         try:
-            h = read_dicom_file(fname, stop_before_pixels=True)
+            h = _read_dicom(fname, stop_before_pixels=True)
         except Exception:
             logger.warning("Doesn't seem to be DICOM, will be skipped: %s", fname)
             continue
@@ -192,7 +267,9 @@ def read_dicoms(path, primary=True, original=True, disable_tqdm=False, read_meta
     vols = []
     for uid in sorted(series):
         items = sorted(series[uid], key=lambda t: t[0][2])          # np.argsort of the z positions (utils.py:211-214)
-        slices = [read_dicom_file(f) for _, f in items]
+        names = [f for _, f in items]
+        slices = [_read_dicom(f) for f in names]
+        _decode_pending(slices, names, device)
         first = slices[0]
         iop = _floats(first.get("ImageOrientationPatient", "1\\0\\0\\0\\1\\0"), 6)
         px = _floats(first.get("PixelSpacing", "1\\1"), 2)           # row spacing (y), column spacing (x)
@@ -334,8 +411,9 @@ def _write_mha(path, arr, like):
         f.write(arr.tobytes())
 
 
-def load_input_image(path, disable_tqdm=False, read_metadata=False):
-    """utils.load_input_image (utils.py:235-269): a file is read as is, a directory as a DICOM series (the largest one)."""
+def load_input_image(path, disable_tqdm=False, read_metadata=False, device=None):
+    """utils.load_input_image (utils.py:235-269): a file is read as is, a directory as a DICOM series (the largest one).
+    `device`: the CUDA device that decodes compressed DICOM (default: LOCAL_RANK, else 0)."""
     if os.path.isfile(path):
         logger.info("Read input: %s", path)
         low = path.lower()
@@ -345,7 +423,7 @@ def load_input_image(path, disable_tqdm=False, read_metadata=False):
             return _read_nifti(path)
         if low.endswith((".mha", ".mhd")):
             return _read_mha(path)
-        h = read_dicom_file(path)                                       # a single DICOM slice
+        h = read_dicom_file(path, device=device)                        # a single DICOM slice
         px = _floats(h.get("PixelSpacing", "1\\1"), 2)
         iop = _floats(h.get("ImageOrientationPatient", "1\\0\\0\\0\\1\\0"), 6)
         rx, ry = np.asarray(iop[:3]), np.asarray(iop[3:])
@@ -357,7 +435,8 @@ def load_input_image(path, disable_tqdm=False, read_metadata=False):
                       tuple(_floats(h.get("ImagePositionPatient", "0\\0\\0"), 3)),
                       tuple(float(x) for x in np.stack([rx, ry, np.cross(rx, ry)], axis=1).ravel()))
     logger.info("Looking for dicoms in %s", path)
-    vols = read_dicoms(path, original=False, primary=False, disable_tqdm=disable_tqdm, read_metadata=read_metadata)
+    vols = read_dicoms(path, original=False, primary=False, disable_tqdm=disable_tqdm, read_metadata=read_metadata,
+                       device=device)
     if len(vols) < 1:
         raise SystemExit("No dicoms found!")
     if len(vols) > 1:
