@@ -9,7 +9,9 @@
                           filled), the frame split over one or more fragments, sequence delimiter
 
 Both encoders are vectorised (bit packing by cumulative code lengths), so a 300 x 512^2 series encodes in seconds.  At
-P = 8 the JPEG encoder is pinned against libjpeg-turbo through Pillow (tests/test_dicom_compressed.py).
+every precision P = 2..16 the JPEG encoder is pinned against libjpeg-turbo (oracle/libjpeg_turbo.py) and against the
+sequential reference decoder oracle/ljpeg_ref.py, and rle_encode against the PackBits reference there
+(tests/test_dicom_compressed.py, tests/test_dicom_conformance.py).
 """
 import heapq
 import struct

@@ -1,7 +1,6 @@
 """Compressed DICOM series (JPEG Lossless .4.57 / .4.70, RLE Lossless .5): the oracle encoders, the encapsulation parser
 and the transfer-syntax handling on the CPU; lm_decode_frames (csrc/decode.cu) bit-exact, batched, on malformed input
 and end to end on the GPU."""
-import io
 import os
 import struct
 
@@ -26,14 +25,22 @@ def _encode(img, syntax, **kw):
 @pytest.mark.parametrize("pt", [0, 2])
 @pytest.mark.parametrize("restart_rows", [0, 3])
 def test_jpeg_encoder_matches_libjpeg_turbo(predictor, pt, restart_rows):
-    Image = pytest.importorskip("PIL.Image")
+    """Every precision P = 2..16 decoded by libjpeg-turbo (Pillow's, through oracle/libjpeg_turbo.py)."""
+    from oracle import libjpeg_turbo as lj
+    if not lj.available():
+        pytest.skip("Pillow's libjpeg-turbo is not installed")
     rng = np.random.default_rng(predictor * 10 + pt + restart_rows)
-    img = rng.integers(0, 256, (19, 23)).astype(np.uint16)
-    img[4:9, 3:] = 255                                           # flat and saturated areas: 0xFF bytes, long zero runs
-    img = (img >> pt) << pt
-    b = dc.jpeg_lossless_encode(img, P=8, predictor=predictor, pt=pt, restart_rows=restart_rows)
-    assert (b"\xff\xdd" in b) == (restart_rows > 0)
-    assert np.array_equal(np.asarray(Image.open(io.BytesIO(b))), img)
+    imgs, streams = [], []
+    for P in range(2, 17):
+        img = rng.integers(0, 1 << P, (19, 23)).astype(np.uint16)
+        img[4:9, 3:] = (1 << P) - 1                              # flat and saturated areas: 0xFF bytes, long zero runs
+        img = (img >> min(pt, P - 1)) << min(pt, P - 1)
+        b = dc.jpeg_lossless_encode(img, P=P, predictor=predictor, pt=min(pt, P - 1), restart_rows=restart_rows)
+        assert (b"\xff\xdd" in b) == (restart_rows > 0)
+        imgs.append(img)
+        streams.append(b)
+    for P, img, (dec, P_read) in zip(range(2, 17), imgs, lj.decode_many_with_header(streams)):
+        assert P_read == P and np.array_equal(dec, img), P
 
 
 @pytest.mark.parametrize("bot", ["empty", "filled"])
@@ -154,6 +161,11 @@ def test_jpeg_roundtrip_predictors(predictor, pt):
     s12 = np.clip(ct, -2048, 2047).astype(np.int16)                 # P = 12 signed: sign extension from bit 11
     _roundtrip_jpeg((s12 >> pt) << pt, True, P=12, predictor=predictor, pt=pt)
     _roundtrip_jpeg((s12 >> pt) << pt, True, P=12, predictor=predictor, pt=pt, restart_rows=1)
+    for P in (2, 8, 12, 15):                                        # unsigned P < 16: no sign extension
+        u = rng.integers(0, 1 << P, (37, 29)).astype(np.uint16)
+        u[:, 5] = (1 << P) - 1
+        _roundtrip_jpeg((u >> min(pt, P - 1)) << min(pt, P - 1), False, P=P, predictor=predictor, pt=min(pt, P - 1),
+                        restart_rows=5 if P % 2 else 0)
 
 
 @gpu
