@@ -193,14 +193,8 @@ LM_API int lm_last_timings(const lm_engine* e, float* ms7, int64_t* kernel_launc
  * stream; read the sum with lm_last_conv_timing after an lm_apply_volume* call), "chunk_kb" (k-blocks
  * accumulated inside the tensor core between fp32 round-to-nearest adds; sets both layer classes),
  * "chunk_kb_wide" (the same for the layers with >= 128 output channels only; defaults: 1 for the 64-channel
- * layers, 2 for the wide ones), "dual_issue" (0/1: a second MMA-issuing thread per CTA on alternate chunks;
- * default 0), "cta_pairs" (0/1: the cta_group::2 convolution kernel: validated, on par, default 0),
- * "weight_mcast" (0 / 2: clusters of two CTAs share every weight stage through TMA multicast),
- * "stem_v2" (0 = first stem kernel, 1 = register-resident, 2 = shared-memory tile, 3 = the same with the next tile's
- * samples fetched one tile ahead, the default; all bit-identical),
- * "graphs" (1, default: a volume's forward - every wave's ~26 launches - is captured once as a CUDA graph and replayed;
- * 0: every kernel is launched individually; per-launch convolution timing and score taps always launch individually),
- * "upsample_v2" (0: one thread per output sample, 1: per cell, 2 = default: per cell with static corner indexing; all bit-identical),
+ * layers, 2 for the wide ones), "graphs" (1, default: a volume's forward - every wave's ~26 launches - is captured
+ * once as a CUDA graph and replayed; 0: every kernel is launched individually; per-launch convolution timing and score taps always launch individually),
  * "merge_ctas" (0, default: the region merge loop of utils.py:310-339 runs on one CTA per SM in batches of independent
  * candidates; 1: the single-CTA sequential loop; n: that many CTAs),
  * "ccl_rule" (1 = pruned neighbour rule of the 26-connected labelling, the default; 0 = probe all 13 backward

@@ -8,7 +8,7 @@
 //
 // GEMM view: M = 128 output pixels (a 16-row x 8-column patch of one image), N = BN output channels,
 // K = taps * Cin walked in k-blocks of BK input channels of one filter tap, BK = one 128-byte row of the operand
-// format (conv_tc.cuh: 64 fp16 or 32 tf32 channels).
+// format (conv_tc.cuh: 64 fp16 channels).
 //   * A operand: ONE 5-D TMA box per BK-channel block - the patch plus its one-pixel halo,
 //     (BK ch, 10 x, 18 y, 2 planes, 1 image) = 180 rows of 128 B per plane - serves all nine taps: the tap
 //     (dy,dx) view is the same shared-memory tile entered at row (dy+1)*10 + (dx+1) with an 8-row-group
@@ -20,7 +20,7 @@
 //   * B operand: one 4-D TMA box (BK cin, BN cout, 1 tap, 2 planes) per k-block.
 //   * both land 128B-swizzled, K-major, i.e. in the canonical tcgen05 shared-memory layout.
 //   * fp32-class accuracy from 11-bit tensor-core operands: every fp32 value is pre-split into a hi and a lo plane
-//     (fp16 hi + fp16 lo * 2^-11 by default, tf32 hi + tf32 lo with LM_OPERAND_F16=0) and each k-step computes
+//     (fp16 hi + fp16 lo * 2^-11) and each k-step computes
 //     hi*hi, hi*lo and lo*hi - three exact products - with TWO instructions: the B tile's hi and lo planes are
 //     adjacent in shared memory, so  A_hi x [B_hi;B_lo]  is one N = 2*BN MMA whose left half of the accumulator is
 //     hi*hi and whose right half is hi*lo; A_lo x B_hi (N = BN) then adds lo*hi into that right half.  The
@@ -32,8 +32,8 @@
 //     are NOT drained per chunk: each ring slot keeps accumulating its corrections for the whole tile (their
 //     drift is 2^-11 times smaller still) and is read once, with the slot's last chunk - so the per-chunk drain
 //     is BN columns, half of the accumulator.
-//   * persistent CTAs (one per SM), warp-specialised: warp 0 TMA producer, warp 1 (and optionally 3) MMA issuer
-//     - one elected lane running mma_issue_loop -, warp 2 TMEM allocator, warps 4-11 epilogue (TMEM lane quarter
+//   * persistent CTAs (one per SM), warp-specialised: warp 0 TMA producer, warp 1 MMA issuer - one elected lane
+//     running mma_issue_loop -, warp 2 TMEM allocator, warps 4-11 epilogue (TMEM lane quarter
 //     = warp % 4, two warps share a quarter and split the columns or, for BN = 64, take alternate tiles).
 #include <atomic>
 #include <stdio.h>
@@ -55,7 +55,7 @@ __device__ unsigned long long g_conv_prof[16];
 #endif
 // LM_EXP: bit mask of timing-only ablations for tools/conv_probe (results are wrong with any bit set):
 //   1 no correction MMAs, 2 chunk drains skip their TMEM loads, 4 tile epilogue skips staging + TMA stores,
-//   8 single MMA issuer, 16 no wide MMAs (only the N = BN correction MMAs), 32 producer loads no weights after the first ring fill
+//   16 no wide MMAs (only the N = BN correction MMAs), 32 producer loads no weights after the first ring fill
 #ifndef LM_EXP
 #define LM_EXP 0
 #endif
@@ -64,35 +64,20 @@ __device__ unsigned long long g_conv_prof[16];
 namespace lm {
 namespace {
 
-#if LM_OPERAND_F16
-#define LM_UMMA_C umma_f16_c
-#define LM_UMMA umma_f16
-#define LM_MAKE_IDESC make_idesc_f16
-#else
-#define LM_UMMA_C umma_tf32_c
-#define LM_UMMA umma_tf32
-#define LM_MAKE_IDESC make_idesc_tf32
-#endif
-
 struct IssueArgs {
-  uint32_t me;     // issuer 0 / 1
   int first_tile, total_tiles, tile_step, num_cb, chunk_kb;
   uint32_t tmem_base, smem_a, smem_b;
   uint32_t full0, empty0, tfull0, tempty0, afull0, aempty0;  // mbarrier arrays (shared-memory addresses)
 };
 
-// The MMA issue loop of one issuer thread.  Chunk g (counted over all tiles of the CTA) lives in accumulator slot
-// g % NBUF and, with two issuers (DUAL), belongs to issuer g & 1; NBUF is even, so every slot is written by one
-// issuer only and the order of additions into each accumulator is fixed (bit-deterministic results).  With DUAL
-// both issuers wait on EVERY weight-stage and activation-buffer barrier in order (a wait that has already
-// completed costs a few instructions) so that their phase bits can never alias; only the owner of a k-block issues
-// its MMAs and releases its weight stage, both release every activation buffer (barrier count 2).
+// The MMA issue loop of the issuer thread.  Chunk g (counted over all tiles of the CTA) lives in accumulator slot
+// g % NBUF.
 //
 // Software pipelining: the tensor pipe's instruction queue is only a few MMAs deep, so the gap between the last MMA
 // of one k-block and the first MMA of the next must stay short.  The barrier waits and ring bookkeeping of k-block
 // i+1 (weight stage, activation buffer) are therefore executed in the MIDDLE of k-block i's MMA burst and the
 // burst's remaining MMAs then follow back to back with k-block i+1's first ones.
-template <int BN, int TAPS, bool DUAL, bool UNROLL = true, int MC = 1>
+template <int BN, int TAPS, bool UNROLL>
 __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
   using C = Cfg<BN>;
   constexpr uint32_t STAGES = C::STAGES, NBUF = C::NBUF;
@@ -100,28 +85,26 @@ __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
   constexpr int PATCH_W = (TAPS == 9) ? HALO_W : TILE_W;  // shared-memory rows per image row of the patch
   constexpr uint32_t A_PLANE = (uint32_t)((TAPS == 9) ? A_PLANE_BYTES_3x3 : A_PLANE_BYTES_1x1) >> 4;
   constexpr uint32_t B_PLANE = (uint32_t)C::B_PLANE_BYTES >> 4;
-  constexpr uint32_t idesc_wide = LM_MAKE_IDESC(BM, 2 * BN), idesc_corr = LM_MAKE_IDESC(BM, BN);
+  constexpr uint32_t idesc_wide = make_idesc_f16(BM, 2 * BN), idesc_corr = make_idesc_f16(BM, BN);
   // shared-memory descriptors as (lo, hi) words: lo = start>>4 | LBO, hi = SBO | version | swizzle.
   // A: K-major SW128 entered at an arbitrary 128-byte row, 8-row group stride = one patch row.
   constexpr uint64_t hi_a = (uint64_t)((uint32_t)((PATCH_W * 128) >> 4) | (1u << 14) | (2u << 29)) << 32;
   constexpr uint64_t hi_b = (uint64_t)((uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29)) << 32;
   const uint32_t a_base_lo = ((g.smem_a & 0x3FFFFu) >> 4) | (1u << 16);
   const uint32_t b_base_lo = ((g.smem_b & 0x3FFFFu) >> 4) | (1u << 16);
-  const uint32_t me = g.me;
   const int num_kb = g.num_cb * TAPS, chunk_kb = g.chunk_kb;
   if (g.first_tile >= g.total_tiles) return;
 
   // state of the k-block whose barriers have been waited for ("current")
   uint32_t s = 0, ph = 0, ab = 0, aph = 0;  // weight ring / activation ring position and phase
-  uint32_t gc = 0;                          // chunks closed by this CTA so far -> slot gc % NBUF, owner gc & 1
+  uint32_t gc = 0;                          // chunks closed by this CTA so far -> slot gc % NBUF
   uint32_t tseq = 0;                        // tiles processed: the epilogue group (BN = 64) of a tile is tseq & 1
   int kc = 0;                               // k-blocks already in the open chunk
   int kb_left = num_kb;                     // k-blocks of the tile still to issue (including the current one)
   uint32_t cit = 0;                         // chunks of this tile already closed
-  auto is_mine = [&](uint32_t chunk) { return !DUAL || ((chunk & 1u) == me); };
   // waits of the first k-block
   mbar_wait(g.afull0, 0);
-  if (is_mine(0)) mbar_wait(g.tempty0, 1);
+  mbar_wait(g.tempty0, 1);
   mbar_wait(g.full0, 0);
 #ifdef LM_CONV_PROFILE
   const long long prof_issue_t0 = clock64();
@@ -137,7 +120,6 @@ __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
       for (int tap = 0; tap < TAPS; ++tap) {
         // tap (dy, dx) = the same patch entered (dy * PATCH_W + dx) rows further (16-byte units: 8 per row)
         const uint32_t tap_off = (TAPS == 9) ? (uint32_t)(((tap / 3) * PATCH_W + (tap % 3)) * 8) : 0u;
-        const bool mine = is_mine(gc);
         const uint32_t buf = gc % NBUF;
         const uint32_t d_tmem = g.tmem_base + buf * (uint32_t)C::ACC_COLS;
         const uint32_t alo = a_cb + tap_off;
@@ -145,20 +127,20 @@ __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
         const bool first = (kc == 0);
         const uint32_t s_cur = s;
         // ---- first part of the burst
-        if (mine) {
+        {
           LM_PROF_T0();
           tc_fence_after();
           if (first) {
             // first k-step of a chunk: hi*hi restarts from zero; the corrections restart only at the slot's first
             // chunk of the tile (cit < NBUF), so the two halves need separate instructions here
-            LM_UMMA_C<false>(d_tmem, hi_a | alo, hi_b | blo, idesc_corr);                              // hi*hi :=
-            LM_UMMA(d_tmem + BN, hi_a | alo, hi_b | (blo + B_PLANE), idesc_corr, cit >= NBUF ? 1u : 0u);  // hi*lo
+            umma_f16_c<false>(d_tmem, hi_a | alo, hi_b | blo, idesc_corr);                              // hi*hi :=
+            umma_f16(d_tmem + BN, hi_a | alo, hi_b | (blo + B_PLANE), idesc_corr, cit >= NBUF ? 1u : 0u);  // hi*lo
           } else {
-            LM_UMMA_C<true>(d_tmem, hi_a | alo, hi_b | blo, idesc_wide);                               // [hi*hi | hi*lo] +=
+            umma_f16_c<true>(d_tmem, hi_a | alo, hi_b | blo, idesc_wide);                               // [hi*hi | hi*lo] +=
           }
-          if (!(LM_EXP & 1)) LM_UMMA_C<true>(d_tmem + BN, hi_a | (alo + A_PLANE), hi_b | blo, idesc_corr);  // lo*hi
-          LM_UMMA_C<true>(d_tmem, hi_a | (alo + 2u), hi_b | (blo + 2u), idesc_wide);
-          if (!(LM_EXP & 1)) LM_UMMA_C<true>(d_tmem + BN, hi_a | (alo + A_PLANE + 2u), hi_b | (blo + 2u), idesc_corr);
+          if (!(LM_EXP & 1)) umma_f16_c<true>(d_tmem + BN, hi_a | (alo + A_PLANE), hi_b | blo, idesc_corr);  // lo*hi
+          umma_f16_c<true>(d_tmem, hi_a | (alo + 2u), hi_b | (blo + 2u), idesc_wide);
+          if (!(LM_EXP & 1)) umma_f16_c<true>(d_tmem + BN, hi_a | (alo + A_PLANE + 2u), hi_b | (blo + 2u), idesc_corr);
           LM_PROF_ADD(10);   // issuing the first two k-steps of the k-block (the thread blocks here when the MMA queue is full)
         }
         // ---- close the bookkeeping of this k-block, advance to the next one and wait for its barriers
@@ -178,28 +160,27 @@ __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
         }
         if (has_next) { LM_PROF_T0(); mbar_wait(g.full0 + 8 * s, ph); LM_PROF_ADD(4); }
         // ---- rest of the burst, then the releases
-        if (mine) {
+        {
           LM_PROF_T0();
 #pragma unroll
           for (int k = 2; k < ROW_BYTES / 32; ++k) {
-            const uint32_t ko = (uint32_t)(k * 2);  // one MMA k-step = 32 B along K (16 fp16 / 8 tf32), >>4
-            LM_UMMA_C<true>(d_tmem, hi_a | (alo + ko), hi_b | (blo + ko), idesc_wide);
-            if (!(LM_EXP & 1)) LM_UMMA_C<true>(d_tmem + BN, hi_a | (alo + A_PLANE + ko), hi_b | (blo + ko), idesc_corr);
+            const uint32_t ko = (uint32_t)(k * 2);  // one MMA k-step = 32 B along K (16 fp16), >>4
+            umma_f16_c<true>(d_tmem, hi_a | (alo + ko), hi_b | (blo + ko), idesc_wide);
+            if (!(LM_EXP & 1)) umma_f16_c<true>(d_tmem + BN, hi_a | (alo + A_PLANE + ko), hi_b | (blo + ko), idesc_corr);
           }
           LM_PROF_ADD(11);   // the other two k-steps
           {
             LM_PROF_T0();
-            if (MC > 1) umma_commit_mcast(g.empty0 + 8 * s_cur, (uint16_t)((1u << MC) - 1u));  // ... in every CTA of the cluster
-            else umma_commit(g.empty0 + 8 * s_cur);      // weight stage consumed (only this issuer read it)
+            umma_commit(g.empty0 + 8 * s_cur);           // weight stage consumed
             if (chunk_end) umma_commit(tfull_cur);       // chunk complete -> the tile's epilogue group may drain it
             LM_PROF_ADD(12);
           }
         }
-        if (tap == TAPS - 1) umma_commit(g.aempty0 + 8 * ab_cur);  // arrives once this issuer's MMAs on the buffer have retired
+        if (tap == TAPS - 1) umma_commit(g.aempty0 + 8 * ab_cur);  // arrives once the MMAs on the buffer have retired
         // the accumulator slot of the next chunk is awaited LAST: with a two-slot ring it is the one hand-shake that
         // regularly blocks (the epilogue drains chunk i-1 while chunk i executes), and blocking in the middle of the
         // burst would leave the tensor pipe with half a k-block queued (measured: 8 % slower on the BN = 128 layers)
-        if (has_next && kc == 0 && is_mine(gc)) { LM_PROF_T0(); mbar_wait(g.tempty0 + 8 * (gc % NBUF), (((gc / NBUF) & 1u) ^ 1u)); LM_PROF_ADD(2); }
+        if (has_next && kc == 0) { LM_PROF_T0(); mbar_wait(g.tempty0 + 8 * (gc % NBUF), (((gc / NBUF) & 1u) ^ 1u)); LM_PROF_ADD(2); }
       }
     }
   }
@@ -208,22 +189,15 @@ __device__ __forceinline__ void mma_issue_loop(const IssueArgs& g) {
 #endif
 }
 
-// MC = 1: independent CTAs.  MC = 2: weight multicast - the two CTAs of a cluster work on two pixel tiles of the SAME
-// output-channel block in lock step per weight stage: CTA r loads plane r (hi / lo) of every stage with a TMA multicast
-// into both CTAs' rings, both CTAs' full barriers count the bytes of both loads, a stage is free again when BOTH issuers'
-// MMAs on it have retired (multicast commit on both CTAs' empty barriers, count 2).  Half the L2 -> SM weight bytes per MAC:
-// the deep layers sit at the chip's L2 throughput cap (DESIGN.md section 4.1).  Everything else - activations, MMAs
-// (cta_group::1), epilogue - is per CTA and unchanged.
-template <int BN, int MC>
+template <int BN>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
-               const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmBX,
-               const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmPool, const ConvParams p) {
+               const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmOut,
+               const __grid_constant__ CUtensorMap tmPool, const ConvParams p) {
   using C = Cfg<BN>;
   constexpr int STAGES = C::STAGES;
   constexpr int NBUF = C::NBUF;
-  constexpr int HALVES = C::HALVES, EGROUPS = C::EGROUPS;
-  constexpr int NC = BN / HALVES;  // accumulator columns held by one epilogue thread (64)
+  constexpr int EGROUPS = C::EGROUPS;
 
   extern __shared__ __align__(1024) uint8_t smem[];   // layout: Cfg<BN> (conv_tc_common.cuh); no static shared memory
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::OFF_BARS);
@@ -241,6 +215,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
   const int tiles_x = p.W / TILE_W, tiles_img = tiles_x * (p.H / TILE_H);
   const int n_tiles = p.Cout / BN;
   const int total_tiles = p.N * tiles_img * n_tiles;
+  const int first_tile = (int)blockIdx.x, tile_step = (int)gridDim.x;   // persistent CTAs walk the tiles round-robin
   const int taps = p.taps;
   const int num_cb = (p.C0 + p.C1) / BK;
   const int num_kb = num_cb * taps;
@@ -248,18 +223,10 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
   const int halo = taps == 9 ? 1 : 0;
   const int chunk_kb = p.chunk_kb;
   const int num_chunks = (num_kb + chunk_kb - 1) / chunk_kb;
-  // Two MMA-issuing warps take alternate chunks unless a chunk spans a whole weight ring (then the issuer that
-  // does not own it could fall a full ring behind and its phase bit would alias); see mma_issue_loop.
-  const bool dual_issue = (MC == 1) && p.dual_issue && (chunk_kb <= STAGES - 1) && (num_chunks >= 2);
-  // work items: tiles (MC = 1) or clusters' tile groups (MC pixel tiles of one channel block, this CTA takes pixel tile
-  // MC * group + rank); every CTA of a cluster walks the same item sequence
-  const uint32_t rank = (MC > 1) ? cluster_ctarank() : 0u;
-  const int first_item = (int)blockIdx.x / MC, item_step = (int)gridDim.x / MC, total_items = total_tiles / MC;
-  auto tile_of = [&](int q) { if (MC == 1) return q; const int mtp = q / n_tiles; return (MC * mtp + (int)rank) * n_tiles + (q - mtp * n_tiles); };
 
   if (warp == 0 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, MC); }
-    for (int s = 0; s < NUM_A_BUFS; ++s) { mbar_init(afull0 + 8 * s, 1); mbar_init(aempty0 + 8 * s, dual_issue ? 2 : 1); }
+    for (int s = 0; s < STAGES; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, 1); }
+    for (int s = 0; s < NUM_A_BUFS; ++s) { mbar_init(afull0 + 8 * s, 1); mbar_init(aempty0 + 8 * s, 1); }
     for (int b = 0; b < EGROUPS * NBUF; ++b) mbar_init(tfull0 + 8 * b, 1);
     for (int b = 0; b < NBUF; ++b) mbar_init(tempty0 + 8 * b, NUM_EPI_THREADS / 32 / EGROUPS);
     fence_mbar_init();
@@ -273,7 +240,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
   }
   tc_fence_before();
   __syncthreads();
-  if (MC > 1) cluster_sync_all();  // the peer's barriers are initialised before any multicast load / commit signals them
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
 #ifdef LM_CONV_PROFILE
@@ -283,30 +249,24 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
   // Both single-issuer roles run as warp-uniform loops (all 32 lanes execute the control flow and poll the
   // barriers, one elected lane issues the TMA / MMA / commit): loop state then lives in uniform registers
   // and the issue thread is not throttled by divergent-code bookkeeping.
-  // Register reallocation (setmaxnreg): warps 0-3 (producer, issuer(s), TMEM allocator) give registers to the two epilogue
-  // warpgroups, whose chunk drains hold 3 x 64 fp32 values per thread: 128 x LM_REGS_LOW + 256 x LM_REGS_HIGH <= 384 x 168.
+  // Register reallocation (setmaxnreg): warps 0-3 (producer, issuer, TMEM allocator) give registers to the two epilogue
+  // warpgroups, whose chunk drains hold 3 x 64 fp32 values per thread: 128 x kRegsLow + 256 x kRegsHigh <= 384 x 168.
   // Each branch starts with its warpgroups' setmaxnreg and the branches only meet again at the kernel's last barrier.
   if (warp >= EPI_WARP0) {
-#if LM_SETMAXNREG
-    setmaxnreg_inc<LM_REGS_HIGH>();
-#endif
+    setmaxnreg_inc<kRegsHigh>();
     // ------------------------------------------------------------------ epilogue warps
-    conv_epilogue_warps<BN, false>(p, &tmOut, &tmPool, tmem_base, tfull0, tempty0, smem_out, reinterpret_cast<float*>(smem + C::OFF_CONST), s_head_w, s_head_b, first_item,
-                                   total_items, item_step, tile_of, num_chunks);
+    conv_epilogue_warps<BN>(p, &tmOut, &tmPool, tmem_base, tfull0, tempty0, smem_out, reinterpret_cast<float*>(smem + C::OFF_CONST), s_head_w, s_head_b,
+                            first_tile, total_tiles, tile_step, num_chunks);
     tc_fence_before();
     __syncthreads();   // the kernel's last barrier (the other warps arrive at it from their own branch)
-    if (MC > 1) cluster_sync_all();
     return;
   } else {
-#if LM_SETMAXNREG
-    setmaxnreg_dec<LM_REGS_LOW>();
-#endif
+    setmaxnreg_dec<kRegsLow>();
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
     uint32_t s = 0, ph = 0, ab = 0, aph = 0;
     const uint32_t a_tx = 2u * (uint32_t)a_plane_bytes;
-    for (int item = first_item; item < total_items; item += item_step) {
-      const int tile = tile_of(item);
+    for (int tile = first_tile; tile < total_tiles; tile += tile_step) {
       const TileCoord t = decode_tile(tile, n_tiles, tiles_x, tiles_img, BN);
       int c = 0;
       for (int cb = 0; cb < num_cb; ++cb, c += BK) {
@@ -323,13 +283,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
         for (int tap = 0; tap < taps; ++tap) {
           { LM_PROF_T0(); mbar_wait(empty0 + 8 * s, ph ^ 1); if (lane == 0) LM_PROF_ADD(1); }
           if (elect_one()) {
-            if ((LM_EXP & 32) && (tile != (int)blockIdx.x || cb > 0 || tap >= STAGES)) {
+            if ((LM_EXP & 32) && (tile != first_tile || cb > 0 || tap >= STAGES)) {
               mbar_arrive(full0 + 8 * s);  // ablation: reuse whatever the stage holds
-            } else if (MC > 1) {
-              // this CTA's plane of the stage, into both CTAs' rings; the local barrier expects both planes
-              mbar_arrive_expect_tx(full0 + 8 * s, C::STAGE_BYTES);
-              tma_load_4d_mcast(smem_u32(smem_b) + s * C::STAGE_BYTES + rank * (uint32_t)C::B_PLANE_BYTES, &tmBX, full0 + 8 * s, c, t.n0, tap,
-                                (int)rank, (uint16_t)((1u << MC) - 1u));
             } else {
               mbar_arrive_expect_tx(full0 + 8 * s, C::STAGE_BYTES);
               tma_load_4d(smem_u32(smem_b) + s * C::STAGE_BYTES, &tmB, full0 + 8 * s, c, t.n0, tap, 0);
@@ -340,34 +295,26 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
         }
       }
     }
-    if (MC > 1) {
-      // cluster tail: the releases of the last STAGES k-blocks (commits from BOTH CTAs' issuers) have landed on this CTA's
-      // barriers before it may exit - no signal is left in flight towards shared memory that a later CTA could own
-      for (int i = 0; i < STAGES; ++i) {
-        mbar_wait(empty0 + 8 * s, ph ^ 1);
-        if (++s == STAGES) { s = 0; ph ^= 1; }
-      }
-    }
-  } else if (warp == 1 || warp == 3) {
-    // ------------------------------------------------------------------ MMA issuers (two warps, one lane each)
+  } else if (warp == 1) {
+    // ------------------------------------------------------------------ MMA issuer (one lane)
     // ncu (profiles/r01_ncu_conv_issuer.md) showed the previous warp-uniform issue loops spending ~60 % of their
     // time in per-k-block bookkeeping (~150 scalar instructions at ~8 cycles each for a lone warp), with the tensor
     // pipe idle meanwhile.  The loop therefore runs in ONE lane, the nine taps are unrolled with compile-time
     // descriptor offsets, and the state per k-block is a ring index, a phase bit and a chunk counter.
     if (elect_one()) {  // (elect.sync, not lane == 0: the compiler then knows the region is single-lane and
                         //  feeds the MMA's uniform-register operands without per-lane broadcast loops)
-      const uint32_t me = (warp == 3) ? 1u : 0u;
-      if (dual_issue || me == 0u) {
-        IssueArgs ia;
-        ia.me = me; ia.first_tile = first_item; ia.total_tiles = total_items; ia.tile_step = item_step;
-        ia.num_cb = num_cb; ia.chunk_kb = chunk_kb; ia.tmem_base = tmem_base;
-        ia.smem_a = smem_u32(smem); ia.smem_b = smem_u32(smem_b);
-        ia.full0 = full0; ia.empty0 = empty0; ia.tfull0 = tfull0; ia.tempty0 = tempty0; ia.afull0 = afull0; ia.aempty0 = aempty0;
-        if (dual_issue) { if (taps == 9) mma_issue_loop<BN, 9, true>(ia); else mma_issue_loop<BN, 1, true>(ia); }
-        else if (taps != 9) mma_issue_loop<BN, 1, false, true, MC>(ia);
-        else if (LM_TAP_LOOP == 2 || (LM_TAP_LOOP == 1 && BN == 64 && num_cb == 1)) mma_issue_loop<BN, 9, false, false, MC>(ia);
-        else mma_issue_loop<BN, 9, false, true, MC>(ia);
-      }
+      IssueArgs ia;
+      ia.first_tile = first_tile; ia.total_tiles = total_tiles; ia.tile_step = tile_step;
+      ia.num_cb = num_cb; ia.chunk_kb = chunk_kb; ia.tmem_base = tmem_base;
+      ia.smem_a = smem_u32(smem); ia.smem_b = smem_u32(smem_b);
+      ia.full0 = full0; ia.empty0 = empty0; ia.tfull0 = tfull0; ia.tempty0 = tempty0; ia.afull0 = afull0; ia.aempty0 = aempty0;
+      // Layers whose tiles are ONE channel block deep (64 input channels: 9 k-blocks per tile) run the nine taps as a real
+      // loop instead of unrolled: these are the layers whose epilogue warps are busy most of the time, and the unrolled
+      // loop's 16 KB of straight-line code then competes with the epilogue's for instruction fetch - measured -22 % / -16 %
+      // on down0.block3 / up3.block3+head, while the 18-k-block up3.block0 is 8 % FASTER unrolled (profiles/r02_call7_*).
+      if (taps != 9) mma_issue_loop<BN, 1, true>(ia);
+      else if (BN == 64 && num_cb == 1) mma_issue_loop<BN, 9, false>(ia);
+      else mma_issue_loop<BN, 9, true>(ia);
     }
     __syncwarp();
   }
@@ -377,7 +324,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
 #ifdef LM_CONV_PROFILE
   if (threadIdx.x == 0) atomicAdd(&g_conv_prof[9], (unsigned long long)(clock64() - prof_kernel_t0));
 #endif
-  if (MC > 1) cluster_sync_all();
   if (warp == 2) {
     tc_fence_after();
     tmem_dealloc(tmem_base, C::TMEM_COLS);
@@ -400,11 +346,7 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-#if LM_OPERAND_F16
 constexpr CUtensorMapDataType kOpType = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-#else
-constexpr CUtensorMapDataType kOpType = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
-#endif
 
 int encode(CUtensorMap* m, CUtensorMapDataType dtype, const void* base, int rank, const cuuint64_t* dims,
            const cuuint64_t* strides, const cuuint32_t* box) {
@@ -433,7 +375,7 @@ int make_conv_maps(ConvMaps* maps, const void* src0, const void* src1, const voi
                    const ConvParams& p, int n_capacity) {
   const cuuint64_t E = kOpBytes;
   if (p.H % TILE_H || p.W % TILE_W || p.C0 % BK || p.C1 % BK || (p.taps != 1 && p.taps != 9)) return -2;
-  const int BN = conv_tile_n(p);
+  const int BN = conv_tile_n(p.Cout);
   if (p.Cout % BN) return -3;
   int r = make_act_map(&maps->a0, src0, n_capacity, p.H, p.W, p.C0, p.taps);
   if (r) return r;
@@ -472,47 +414,25 @@ int make_conv_maps(ConvMaps* maps, const void* src0, const void* src1, const voi
   cuuint64_t dims[4] = {(cuuint64_t)Cin, (cuuint64_t)p.Cout, (cuuint64_t)p.taps, 2};
   cuuint64_t strides[3] = {(cuuint64_t)Cin * E, (cuuint64_t)p.Cout * Cin * E, (cuuint64_t)p.taps * p.Cout * Cin * E};
   cuuint32_t box[4] = {BK, (cuuint32_t)BN, 1, 2};
-  r = encode(&maps->b, kOpType, weights, 4, dims, strides, box);
-  if (r) return r;
-  // weight boxes of the CTA-pair kernel (optional: a failure only disables that kernel)
-  cuuint32_t box_x[4] = {BK, (cuuint32_t)BN, 1, 1}, box_yw[4] = {BK, (cuuint32_t)(BN / 2), 1, 2};
-  maps->pair_ok = (encode(&maps->bx, kOpType, weights, 4, dims, strides, box_x) == 0 &&
-                   encode(&maps->byw, kOpType, weights, 4, dims, strides, box_yw) == 0) ? 1 : 0;
-  return 0;
+  return encode(&maps->b, kOpType, weights, 4, dims, strides, box);
 }
 
-template <int BN, int MC>
+template <int BN>
 static int launch_impl(const ConvMaps& maps, const ConvParams& p, int num_sms, cudaStream_t stream) {
   // the opt-in to > 48 KB of dynamic shared memory is a per-device function attribute
   static std::atomic<unsigned long long> attr_set_mask{0ull};  // engines of several host threads may launch concurrently
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return -9;
   if (!((attr_set_mask.load(std::memory_order_acquire) >> dev) & 1ull)) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<BN, MC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          Cfg<BN>::DYN_SMEM);
     if (e != cudaSuccess) return (int)e;
     attr_set_mask.fetch_or(1ull << dev, std::memory_order_release);
   }
   const int total = p.N * (p.H / TILE_H) * (p.W / TILE_W) * (p.Cout / BN);
-  if (MC == 1) {
-    const int grid = total < num_sms ? total : num_sms;
-    conv_tc_kernel<BN, 1><<<grid, NUM_THREADS, Cfg<BN>::DYN_SMEM, stream>>>(maps.a0, maps.a1, maps.b, maps.bx, maps.out, maps.pool, p);
-    return (int)cudaGetLastError();
-  }
-  // clusters of MC CTAs: MC pixel tiles of one channel block per work item (every level has an even number of pixel tiles)
-  const int groups = total / MC, sm_groups = num_sms / MC;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(MC * (groups < sm_groups ? groups : sm_groups)), 1, 1);
-  cfg.blockDim = dim3(NUM_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = Cfg<BN>::DYN_SMEM;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = MC; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, conv_tc_kernel<BN, MC>, maps.a0, maps.a1, maps.b, maps.bx, maps.out, maps.pool, p);
-  return (int)(e != cudaSuccess ? e : cudaGetLastError());
+  const int grid = total < num_sms ? total : num_sms;
+  conv_tc_kernel<BN><<<grid, NUM_THREADS, Cfg<BN>::DYN_SMEM, stream>>>(maps.a0, maps.a1, maps.b, maps.out, maps.pool, p);
+  return (int)cudaGetLastError();
 }
 
 #ifdef LM_CONV_PROFILE
@@ -523,20 +443,16 @@ void conv_prof_read(unsigned long long* out) { cudaMemcpyFromSymbol(out, g_conv_
 // Sets the kernels' > 48 KB dynamic shared-memory opt-in on the current device (lm_create calls it, so that no launch -
 // in particular none inside a CUDA-graph capture - has to).
 int conv_tc_prepare() {
-  cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<128, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128>::DYN_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<64, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<64>::DYN_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<128, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128>::DYN_SMEM);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<64, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<64>::DYN_SMEM);
+  cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128>::DYN_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_tc_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<64>::DYN_SMEM);
   return (int)e;
 }
 
 int launch_conv_tc(const ConvMaps& maps, const ConvParams& p, int num_sms, cudaStream_t stream) {
   if (p.mode == kModeHead && (p.Cout != 64 || p.K > MAX_CLASSES)) return -4;
   if (p.chunk_kb < 1) return -5;
-  if (p.weight_mcast == 2)
-    return conv_tile_n(p) == 128 ? launch_impl<128, 2>(maps, p, num_sms, stream) : launch_impl<64, 2>(maps, p, num_sms, stream);
-  return conv_tile_n(p) == 128 ? launch_impl<128, 1>(maps, p, num_sms, stream)
-                               : launch_impl<64, 1>(maps, p, num_sms, stream);
+  return conv_tile_n(p.Cout) == 128 ? launch_impl<128>(maps, p, num_sms, stream)
+                                    : launch_impl<64>(maps, p, num_sms, stream);
 }
 
 }  // namespace lm

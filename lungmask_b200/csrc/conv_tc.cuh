@@ -5,33 +5,21 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// Operand format of the tensor-core convolutions (compile-time, one format per build):
-//   1 (default)  fp16 pairs, tcgen05 kind::f16:  x = hi + lo * 2^-11, hi = fp16(x), lo = fp16((x - hi) * 2^11).
-//                Both halves carry 11 significant bits (as tf32 does), every product is exact in fp32, and an
-//                MMA instruction covers K = 16 at the rate kind::tf32 covers K = 8: the 3-product scheme runs
-//                at twice the tf32 rate and moves half the bytes.  The scaled low half keeps the residuals
-//                of small values out of the fp16 subnormal range; the hi*lo + lo*hi accumulator is multiplied
-//                by 2^-11 when it is read.  fp16 saturates at 65504: the epilogues raise ConvParams::range_flag
-//                when a value leaves that range; the engine then lowers that tensor's power-of-two scale
-//                (ConvParams::out_scale) and runs the forward again - exact, and never a wrong mask.
-//   0            tf32 pairs, kind::tf32 (round 1's first scheme; no range limit, half the throughput).
-#ifndef LM_OPERAND_F16
-#define LM_OPERAND_F16 1
-#endif
+// Operand format of the tensor-core convolutions: fp16 pairs, tcgen05 kind::f16:  x = hi + lo * 2^-11, hi = fp16(x),
+// lo = fp16((x - hi) * 2^11).  Both halves carry 11 significant bits (as tf32 does), every product is exact in fp32, and an
+// MMA instruction covers K = 16 at the rate kind::tf32 covers K = 8: the 3-product scheme runs at twice the tf32 rate and
+// moves half the bytes.  The scaled low half keeps the residuals of small values out of the fp16 subnormal range; the
+// hi*lo + lo*hi accumulator is multiplied by 2^-11 when it is read.  fp16 saturates at 65504: the epilogues raise
+// ConvParams::range_flag when a value leaves that range; the engine then lowers that tensor's power-of-two scale
+// (ConvParams::out_scale) and runs the forward again - exact, and never a wrong mask.
 
 namespace lm {
 
-#if LM_OPERAND_F16
 using op_t = __half;
 constexpr float kLoScale = 2048.f, kLoUnscale = 1.f / 2048.f;
 constexpr float kOpMax = 65504.f;
-#else
-using op_t = float;
-constexpr float kLoScale = 1.f, kLoUnscale = 1.f;
-constexpr float kOpMax = 3.0e38f;
-#endif
 constexpr int kOpBytes = (int)sizeof(op_t);
-constexpr int kBK = 128 / kOpBytes;  // input channels per k-block: one 128-byte swizzle row (64 fp16 / 32 tf32)
+constexpr int kBK = 128 / kOpBytes;  // input channels per k-block: one 128-byte swizzle row (64 fp16)
 
 // Activation tensors feeding / produced by the tensor-core convolutions are "split planes":
 //   [N][2][H][W][C] op_t, plane 0 = hi, plane 1 = lo (scaled by kLoScale), so that hi + lo * kLoUnscale
@@ -53,16 +41,12 @@ struct ConvParams {
   int mode;           // ConvMode
   int chunk_kb;       // k-blocks (kBK channels x 1 tap) accumulated inside the tensor core before the
                       // partial sum is added, round-to-nearest, into fp32 registers
-  int dual_issue;     // 1: two MMA-issuing threads take alternate chunks (0: one issuer)
-  int weight_mcast;   // 2: clusters of two CTAs share every weight stage through TMA multicast (conv_tc.cu, MC = 2); 0 / 1: off
-  int tile_n;         // output-channel tile: 0 = conv_tile_n(Cout); 64 forces the BN = 64 kernel (two epilogue groups on
-                      // alternate tiles) for a layer with Cout >= 128 - must be set before make_conv_maps
   const float* bias;  // [Cout]
   const float* scale; // [Cout]  folded BN:  y = relu(.) * scale + shift
   const float* shift; // [Cout]
   void* out;          // mode 0/1: op_t [N][2][H][W][Cout]; mode 2: fp32 [N][H][W][Cout]; mode 3: unused
   void* out_pool;     // mode 1: op_t [N][2][H/2][W/2][Cout]
-  int* range_flag;    // set to 1 when an output leaves the operand format's range (fp16 build); may be nullptr
+  int* range_flag;    // set to 1 when an output leaves the operand format's range; may be nullptr
   // Power-of-two range management (exact: a power of two changes no significand).  The operand planes of a tensor hold
   // value * act_scale, weights hold w * w_scale; the epilogue multiplies the accumulator by in_unscale =
   // 1 / (act_scale(in) * w_scale) before the bias and stores y * out_scale.  All 1.0 unless the engine had to move a
@@ -79,10 +63,6 @@ struct ConvParams {
 struct ConvMaps {
   CUtensorMap a0, a1, b;
   CUtensorMap out, pool;  // TMA-store maps of the output tile (mode 0/1/2) and of the pooled tile (mode 1)
-  // weight boxes of the CTA-pair kernel (conv_tc_pair.cu): bx = (BK cin, BN cout, 1 tap, 1 plane),
-  // byw = (BK cin, BN/2 cout, 1 tap, 2 planes); pair_ok = both were encoded
-  CUtensorMap bx, byw;
-  int pair_ok;
 };
 
 // Builds the TMA descriptors. src1 may be nullptr when C1 == 0. Returns 0 on success.
@@ -92,15 +72,10 @@ int make_conv_maps(ConvMaps* maps, const void* src0, const void* src1, const voi
 // Launches the convolution on `stream`. Returns a cudaError_t value (0 = ok).
 int launch_conv_tc(const ConvMaps& maps, const ConvParams& p, int num_sms, cudaStream_t stream);
 
-// CTA-pair variant (conv_tc_pair.cu, tcgen05 cta_group::2; experimental, see the file header). Same contract.
-int launch_conv_tc_pair(const ConvMaps& maps, const ConvParams& p, int num_sms, cudaStream_t stream);
-
-// Per-device preparation (dynamic shared-memory opt-in of every kernel variant); returns a cudaError_t value.
+// Per-device preparation (dynamic shared-memory opt-in of both kernel instantiations); returns a cudaError_t value.
 int conv_tc_prepare();
-int conv_tc_pair_prepare();
 
 // BN (output-channel tile) chosen for a given Cout.
 inline int conv_tile_n(int cout) { return cout >= 128 ? 128 : 64; }
-inline int conv_tile_n(const ConvParams& p) { return p.tile_n == 64 ? 64 : conv_tile_n(p.Cout); }
 
 }  // namespace lm

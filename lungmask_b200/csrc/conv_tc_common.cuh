@@ -1,39 +1,22 @@
-// Shared pieces of the tensor-core convolution kernels (conv_tc.cu: one CTA per tile, conv_tc_pair.cu: CTA pairs with
-// tcgen05 cta_group::2): tile geometry, shared-memory budget and the epilogue warps' code - chunk drains out of TMEM
-// with round-to-nearest fp32 accumulation, then bias / ReLU / BatchNorm, operand-plane split, 2x2 average pool, 1x1 head
-// with log-softmax + argmax, and the TMA stores.  One copy, so that both kernels produce the same bits by construction.
+// Pieces of the tensor-core convolution kernel (conv_tc.cu): tile geometry, shared-memory budget and the epilogue warps'
+// code - chunk drains out of TMEM with round-to-nearest fp32 accumulation, then bias / ReLU / BatchNorm, operand-plane split,
+// 2x2 average pool, 1x1 head with log-softmax + argmax, and the TMA stores.
 // The including file defines LM_PROF_T0 / LM_PROF_ADD / LM_EXP (instrumentation of tools/conv_probe) first.
+// Staged rows leave through cp.async.bulk.tensor stores out of a 4 KB buffer per epilogue warp.  (Round 2 measured coalesced
+// 16-byte stores out of the same buffer: equal within 0.5 % per wave, profiles/r02_call5_summary.md; 8-row staging passes with a
+// fourth weight stage: 3.4 % slower; and an L1 prefetch of the per-channel constants: no gain, superseded by the shared-memory
+// copy below.)
 #pragma once
-#ifndef LM_TMA_STORES
-// 1 (default): staged rows leave through cp.async.bulk.tensor stores out of a 4 KB buffer per epilogue warp.
-// 2: coalesced 16-byte stores in ONE sweep out of the same buffer: equal within 0.5 % per wave (5 % faster on the pooled
-//    level-0 layer, 4 % slower on the two other 256 x 256 layers; profiles/r02_call5_summary.md).
-// (Round 2 also measured 8-row staging passes with a fourth weight stage: 3.4 % slower, removed; and an L1 prefetch of the
-//  per-channel constants: no gain, superseded by the shared-memory copy below.)
-#define LM_TMA_STORES 1
-#endif
-#ifndef LM_SETMAXNREG
-#define LM_SETMAXNREG 1
-#endif
-#ifndef LM_REGS_LOW
-#define LM_REGS_LOW 88
-#define LM_REGS_HIGH 208
-#endif
-#ifndef LM_TAP_LOOP
-// Layers whose tiles are ONE channel block deep (64 input channels: 9 k-blocks per tile) run the issue loop with the nine taps
-// as a real loop instead of unrolled: these are the layers whose epilogue warps are busy most of the time, and the unrolled
-// loop's 16 KB of straight-line code then competes with the epilogue's for instruction fetch - measured -22 % / -16 % on
-// down0.block3 / up3.block3+head, while the 18-k-block up3.block0 is 8 % FASTER unrolled (profiles/r02_call7_*).
-// 0 = always unrolled, 1 = this rule, 2 = always a loop.
-#define LM_TAP_LOOP 1
-#endif
 #include "conv_tc.cuh"
 #include "sm100_ptx.cuh"
 
 namespace lm {
 namespace {
 
-constexpr int BM = 128, BK = kBK, TILE_H = 16, TILE_W = 8;  // BK channels = one 128-byte row (64 fp16 / 32 tf32)
+// setmaxnreg budgets: warps 0-3 (producer, issuer, TMEM allocator) give registers to the two epilogue warpgroups
+constexpr int kRegsLow = 88, kRegsHigh = 208;
+
+constexpr int BM = 128, BK = kBK, TILE_H = 16, TILE_W = 8;  // BK channels = one 128-byte row (64 fp16)
 constexpr int ROW_BYTES = 128;
 constexpr int HALO_W = TILE_W + 2, HALO_H = TILE_H + 2;
 constexpr int A_PLANE_BYTES_3x3 = HALO_W * HALO_H * ROW_BYTES;  // 180 rows x 128 B = 23040 B per plane
@@ -93,14 +76,12 @@ __device__ __forceinline__ TileCoord decode_tile(int tile, int n_tiles, int tile
   return t;
 }
 
-// The epilogue warps (warps EPI_WARP0 .. EPI_WARP0 + 7) of one CTA.  Work items first_item, first_item + item_step, ...
-// < total_items map to tiles through tile_of(item) (identity for the single-CTA kernel, the CTA's half of a tile pair for
-// the pair kernel).  PAIR: "accumulator drained" is signalled on the pair leader's barrier.
-template <int BN, bool PAIR, typename TileOf>
+// The epilogue warps (warps EPI_WARP0 .. EPI_WARP0 + 7) of one CTA: tiles first_tile, first_tile + tile_step, ... < total_tiles.
+template <int BN>
 __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const CUtensorMap* tmOut, const CUtensorMap* tmPool,
                                                     uint32_t tmem_base, uint32_t tfull0, uint32_t tempty0, uint8_t* smem_out,
-                                                    float* smem_const, const float* s_head_w, const float* s_head_b, int first_item,
-                                                    int total_items, int item_step, TileOf tile_of, int num_chunks) {
+                                                    float* smem_const, const float* s_head_w, const float* s_head_b, int first_tile,
+                                                    int total_tiles, int tile_step, int num_chunks) {
   using C = Cfg<BN>;
   constexpr int NBUF = C::NBUF;
   constexpr int HALVES = C::HALVES, EGROUPS = C::EGROUPS;
@@ -120,9 +101,9 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
   static_assert(NC == 64, "one epilogue thread holds 64 accumulator columns");
   float* cst = smem_const + (warp - EPI_WARP0) * CONST_WARP_FLOATS;   // this warp's bias | scale | shift (64 floats each)
   int const_n0 = -1;                                                  // channel block they belong to
-  for (int item = first_item; item < total_items; item += item_step, ++tseq) {
+  for (int tile = first_tile; tile < total_tiles; tile += tile_step, ++tseq) {
     if (EGROUPS == 2 && (tseq & 1u) != egroup) { buf = (buf + (uint32_t)num_chunks) % NBUF; continue; }  // the other group's tile
-    const TileCoord t = decode_tile(tile_of(item), n_tiles, tiles_x, tiles_img, BN);
+    const TileCoord t = decode_tile(tile, n_tiles, tiles_x, tiles_img, BN);
     float acc[NC];
 #pragma unroll
     for (int i = 0; i < NC; ++i) acc[i] = 0.f;
@@ -161,7 +142,7 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
       auto hand_back = [&]() {
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) { if (PAIR) mbar_arrive_leader(tempty0 + 8 * buf); else mbar_arrive(tempty0 + 8 * buf); }
+        if (lane == 0) mbar_arrive(tempty0 + 8 * buf);
       };
       // all TMEM reads of this slot first, then hand the slot back BEFORE the register adds: the
       // tensor core's next chunk on this slot does not have to wait for the fp32 accumulation
@@ -221,20 +202,9 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
     };
     // one 128-byte row of operand-format channels (BK of them) per plane, from fp32 values: both planes in one pass
     auto pack_rows = [&](const float* src, uint32_t* vh, uint32_t* vl) {
-#if LM_OPERAND_F16
 #pragma unroll
       for (int i = 0; i < 32; ++i) split_f16x2(src[2 * i], src[2 * i + 1], vh[i], vl[i]);
-#else
-#pragma unroll
-      for (int i = 0; i < 32; ++i) {
-        float hi, lo;
-        split_tf32(src[i], hi, lo);
-        vh[i] = __float_as_uint(hi);
-        vl[i] = __float_as_uint(lo);
-      }
-#endif
     };
-#if LM_TMA_STORES == 1
     auto round_begin = [&]() {
       if (issuer) tma_store_wait_read();  // this warp's previous store has finished reading the buffer
       __syncwarp();
@@ -243,45 +213,6 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
       fence_proxy_async();
       __syncwarp();
     };
-#else
-    // LM_TMA_STORES == 2: the staged rows leave with plain 16-byte stores - lanes 8m .. 8m+7 read the eight pieces of one
-    // 128-byte row (one pixel's channel group: a full line of the channels-last tensor), so every warp instruction writes
-    // four complete lines.  flush8: staged rows m and m + 4 -> `dst` and `dst + step` (the warp's 8 pooled pixels are one call).
-    auto flush8 = [&](uint8_t* dst, size_t step) {
-      const uint32_t m = (uint32_t)lane >> 3, piece = (uint32_t)lane & 7u;
-      uint4 v0, v1;
-      const uint32_t a0 = stage + m * 128u + ((piece ^ m) << 4), a1 = stage + (m + 4u) * 128u + ((piece ^ (m + 4u)) << 4);
-      asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v0.x), "=r"(v0.y), "=r"(v0.z), "=r"(v0.w) : "r"(a0) : "memory");
-      asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v1.x), "=r"(v1.y), "=r"(v1.z), "=r"(v1.w) : "r"(a1) : "memory");
-      *reinterpret_cast<uint4*>(dst) = v0;
-      *reinterpret_cast<uint4*>(dst + step) = v1;
-    };
-    // emit32: this lane's 128-byte row (its pixel, one channel group of one plane) -> global.  The warp's 32 pixels are 4
-    // image rows of 8.  `img` = first byte of the (image, plane) in the channels-last tensor, cpix = bytes per pixel,
-    // c0 = channel offset in bytes.
-    auto emit32 = [&](const uint32_t* v, uint8_t* img, uint32_t cpix, uint32_t c0) {
-      uint8_t* dst = img + ((size_t)ty0 * p.W + t.x0 + (lane >> 3)) * cpix + c0 + (lane & 7) * 16;
-      const size_t pitch = (size_t)p.W * cpix;
-      // the whole 32-pixel plane is staged at once (4 KB per warp, as for the TMA stores) and leaves in one sweep
-      __syncwarp();
-      stage_row((uint32_t)lane, v);
-      __syncwarp();
-      {
-        const uint32_t m = (uint32_t)lane >> 3, piece = (uint32_t)lane & 7u;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {                      // image row k of the warp's four: staged rows 8k + m and 8k + 4 + m
-          uint4 v0, v1;
-          const uint32_t r0 = 8u * k + m, r1 = r0 + 4u;
-          const uint32_t a0 = stage + r0 * 128u + ((piece ^ (r0 & 7u)) << 4), a1 = stage + r1 * 128u + ((piece ^ (r1 & 7u)) << 4);
-          asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v0.x), "=r"(v0.y), "=r"(v0.z), "=r"(v0.w) : "r"(a0) : "memory");
-          asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v1.x), "=r"(v1.y), "=r"(v1.z), "=r"(v1.w) : "r"(a1) : "memory");
-          *reinterpret_cast<uint4*>(dst) = v0;
-          *reinterpret_cast<uint4*>(dst + (size_t)4 * cpix) = v1;
-          dst += pitch;
-        }
-      }
-    };
-#endif
 
     if (p.mode == kModeLinear) {
 #pragma unroll
@@ -293,15 +224,10 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
           v[4 * i] = __float_as_uint(__fmaf_rn(acc[g * 32 + 4 * i], unscale, b.x)); v[4 * i + 1] = __float_as_uint(__fmaf_rn(acc[g * 32 + 4 * i + 1], unscale, b.y));
           v[4 * i + 2] = __float_as_uint(__fmaf_rn(acc[g * 32 + 4 * i + 2], unscale, b.z)); v[4 * i + 3] = __float_as_uint(__fmaf_rn(acc[g * 32 + 4 * i + 3], unscale, b.w));
         }
-#if LM_TMA_STORES == 1
         round_begin();
         stage_row((uint32_t)lane, v);
         round_end();
         if (issuer && !(LM_EXP & 4)) { tma_store_4d(tmOut, stage, cbase + g * F32_ROW_CH, t.x0, ty0, t.n); tma_store_commit(); }
-#else
-        if (!(LM_EXP & 4))
-          emit32(v, static_cast<uint8_t*>(p.out) + (size_t)t.n * p.H * p.W * p.Cout * 4, (uint32_t)p.Cout * 4u, (uint32_t)(cbase + g * F32_ROW_CH) * 4u);
-#endif
       }
     } else {
       const float4* scale4 = bias4 + NC / 4;
@@ -346,14 +272,12 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
         p.labels[((size_t)t.n * p.H + y) * p.W + x] = (uint8_t)best;
       } else {
         // (the stored planes hold y * out_scale: the power-of-two factor is already in the scale / shift copies)
-#if LM_OPERAND_F16
         {  // fp16 saturates: report instead of storing inf (the engine lowers out_scale and runs again)
           bool ovf = false;
 #pragma unroll
           for (int i = 0; i < NC; ++i) ovf |= !(fabsf(acc[i]) <= kOpMax);
           if (__any_sync(0xffffffffu, ovf) && lane == 0 && p.range_flag) *p.range_flag = 1;
         }
-#endif
 #pragma unroll
         for (int g = 0; g < NC / BK; ++g) {
           uint32_t vh[32], vl[32];
@@ -361,16 +285,10 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
 #pragma unroll
           for (int plane = 0; plane < 2; ++plane) {
             const uint32_t* v = plane ? vl : vh;
-#if LM_TMA_STORES == 1
             round_begin();
             stage_row((uint32_t)lane, v);
             round_end();
             if (issuer && !(LM_EXP & 4)) { tma_store_5d(tmOut, stage, cbase + g * BK, t.x0, ty0, plane, t.n); tma_store_commit(); }
-#else
-            if (!(LM_EXP & 4))
-              emit32(v, static_cast<uint8_t*>(p.out) + ((size_t)t.n * 2 + plane) * p.H * p.W * p.Cout * kOpBytes, (uint32_t)(p.Cout * kOpBytes),
-                     (uint32_t)((cbase + g * BK) * kOpBytes));
-#endif
           }
         }
         if (p.mode == kModeReluBnPool) {
@@ -392,24 +310,10 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
 #pragma unroll
             for (int plane = 0; plane < 2; ++plane) {
               const uint32_t* v = plane ? vl : vh;
-#if LM_TMA_STORES == 1
               round_begin();
               if (writer) stage_row(prow, v);
               round_end();
               if (issuer && !(LM_EXP & 4)) { tma_store_5d(tmPool, stage, cbase + g * BK, t.x0 >> 1, ty0 >> 1, plane, t.n); tma_store_commit(); }
-#else
-              if (!(LM_EXP & 4)) {   // the warp's 8 pooled pixels (2 rows x 4) are one pass
-                __syncwarp();
-                if (writer) stage_row(prow, v);
-                __syncwarp();
-                // staged rows 0..3 = pooled row ty0/2, rows 4..7 = the next pooled row: row m and m + 4 are one image row apart
-                const uint32_t cpix = (uint32_t)(p.Cout * kOpBytes);
-                const int Wp = p.W / 2;
-                uint8_t* img = static_cast<uint8_t*>(p.out_pool) + ((size_t)t.n * 2 + plane) * (p.H / 2) * Wp * cpix;
-                flush8(img + ((size_t)(ty0 >> 1) * Wp + (t.x0 >> 1) + (lane >> 3)) * cpix + (uint32_t)((cbase + g * BK) * kOpBytes) + (lane & 7) * 16,
-                       (size_t)Wp * cpix);
-              }
-#endif
             }
           }
         }
@@ -417,9 +321,7 @@ __device__ __forceinline__ void conv_epilogue_warps(const ConvParams& p, const C
     }
     if (warp == EPI_WARP0 && lane == 0) LM_PROF_ADD(8);
   }
-#if LM_TMA_STORES == 1
   if (lane == 0) tma_store_wait_all();  // every epilogue warp's issuer: global writes complete before exit
-#endif
 }
 
 }  // namespace

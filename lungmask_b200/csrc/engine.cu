@@ -198,16 +198,6 @@ struct lm_engine {
   uint64_t graph_epoch = 1;
   int use_graphs = 1;     // 0: launch every kernel individually (also whenever per-launch conv timing or score taps are on)
   int64_t graph_launches = 0, graph_hits = 0;
-  unsigned bn64_mask = 0; // bit i: layer i of LAYERS uses BN = 64 output-channel tiles although Cout >= 128 (read at lm_load_weights)
-  int dual_issue = 0;     // 1: two MMA-issuing threads per CTA on alternate chunks (conv_tc.cu)
-  int weight_mcast = 0;   // 2: clusters of two CTAs share each weight stage through TMA multicast (conv_tc.cu, MC = 2)
-  int cta_pairs = 0;      // 1: the cta_group::2 kernel (conv_tc_pair.cu): bit-identical on hardware, but slower than one CTA per tile
-                          //    so far (r02: 14.3 vs 8.7 ms per 37-slice wave, profiles/r02_*) - opt-in
-  int stem_v2 = 3;        // stem kernel version: 0 stem_kernel, 1 stem_kernel_v2 - weights in registers, 4-pixel quads
-                          // (bit-identical to stem_kernel, r02 GPU tests), 2 stem_kernel_v3 - shared input tile and weights,
-                          // 3 (default) stem_kernel_v3 with the next tile's samples fetched one tile ahead
-  int upsample_v2 = 2;    // 2 (default): upsample2x_cells_kernel<true> - one load per output sample, corners indexed statically;
-                          // 1: the same with run-time corner selection, 0: upsample2x_kernel (all three bit-identical)
   int chunk_kb = 1;       // k-blocks per TMEM chunk for the 64-channel layers (ring of 4 slots)
   int chunk_kb_wide = 2;  // ... for the layers with Cout >= 128 (ring of 2 slots: chunk 1 leaves the tensor pipe waiting
                           // for the drain; chunk 2 costs < 1e-5 of score accuracy there, tools/debug_gpu.py)
@@ -258,10 +248,10 @@ int forward_batch(lm_engine* e, Slot& s, const void* d_in, bool in_f32, int n, u
   int* const range = e->d_range + (size_t)(&s - e->slots) * RANGE_STRIDE;
   if (in_f32)
     RC(launch_stem_f32(static_cast<const float*>(d_in), e->act[A0], s.stem_w, s.stem_bias, s.stem_scale, s.stem_shift, n, R, R,
-                       range + A0, s.act_scale[A0], e->stem_v2, e->num_sms, e->st));
+                       range + A0, s.act_scale[A0], e->num_sms, e->st));
   else
-    RC(launch_stem_any(static_cast<const int16_t*>(d_in), e->act[A0], s.stem_w, s.stem_bias, s.stem_scale, s.stem_shift, n, R, R,
-                       range + A0, s.act_scale[A0], e->stem_v2, e->num_sms, e->st));
+    RC(launch_stem(static_cast<const int16_t*>(d_in), e->act[A0], s.stem_w, s.stem_bias, s.stem_scale, s.stem_shift, n, R, R,
+                   range + A0, s.act_scale[A0], e->num_sms, e->st));
   e->launches++;
   int up = 0;
   for (int i = 0; i < NUM_LAYERS; ++i) {
@@ -272,8 +262,6 @@ int forward_batch(lm_engine* e, Slot& s, const void* d_in, bool in_f32, int n, u
     p.range_flag = L.dst >= 0 ? range + L.dst : nullptr;
     p.in_unscale = 1.f / (s.act_scale[L.src0] * s.lw[i].w_scale);   // src1 (virtual concat) shares src0's scale group
     p.out_scale = (L.mode == kModeReluBn || L.mode == kModeReluBnPool) ? s.act_scale[L.dst] : 1.f;
-    p.dual_issue = e->dual_issue;
-    p.weight_mcast = (e->weight_mcast == 2 && s.maps[i].pair_ok) ? 2 : 0;
     if (p.mode == kModeHead) { p.labels = d_labels; p.scores = d_scores; }
     if (time_convs) {
       if (e->ev_used + 2 > e->ev_pool.size()) {
@@ -281,15 +269,13 @@ int forward_batch(lm_engine* e, Slot& s, const void* d_in, bool in_f32, int n, u
       }
       cudaEventRecord(e->ev_pool[e->ev_used], e->st);
     }
-    RC(e->cta_pairs ? launch_conv_tc_pair(s.maps[i], p, e->num_sms, e->st) : launch_conv_tc(s.maps[i], p, e->num_sms, e->st));
+    RC(launch_conv_tc(s.maps[i], p, e->num_sms, e->st));
     if (time_convs) { cudaEventRecord(e->ev_pool[e->ev_used + 1], e->st); e->ev_used += 2; }
     e->launches++;
     if (up < 4 && UPS[up].after_layer == i) {
       const ActSpec& src = ACT[UPS[up].src];
-      RC((e->upsample_v2 >= 2 ? launch_upsample2x_cells_static : e->upsample_v2 ? launch_upsample2x_cells : launch_upsample2x)(
-          static_cast<const float*>(e->act[UPS[up].src]), e->act[UPS[up].dst], n,
-                                                                      R >> src.level, R >> src.level, src.C, range + UPS[up].dst,
-                                                                      s.act_scale[UPS[up].dst], e->num_sms, e->st));
+      RC(launch_upsample2x(static_cast<const float*>(e->act[UPS[up].src]), e->act[UPS[up].dst], n, R >> src.level, R >> src.level, src.C,
+                           range + UPS[up].dst, s.act_scale[UPS[up].dst], e->num_sms, e->st));
       e->launches++;
       ++up;
     }
@@ -462,7 +448,7 @@ int range_finish(lm_engine* e) {
   if (weight_flag || give_up) {
     e->range_retries = 0;
     return fail(LM_ERR_RANGE, "an activation exceeded the fp16 operand range even after rescaling by 2^-32 (|x| > 2.8e14): "
-                              "the weights are not a usable network (rebuild with -DLM_OPERAND_F16=0 for tf32 operands)");
+                              "the weights are not a usable network");
   }
   return 1;
 }
@@ -640,18 +626,11 @@ int lm_create(int device, int batch_capacity, lm_engine** out) {
 static int create_resources(lm_engine* e) {
   const int batch_capacity = e->B;
   if (const char* c = getenv("LM_CHUNK_KB")) { int v = atoi(c); if (v >= 1) e->chunk_kb = e->chunk_kb_wide = v; }
-  if (const char* c = getenv("LM_DUAL_ISSUE")) e->dual_issue = atoi(c) != 0;
-  if (const char* c = getenv("LM_CTA_PAIRS")) e->cta_pairs = atoi(c) != 0;
-  if (const char* c = getenv("LM_WEIGHT_MCAST")) e->weight_mcast = atoi(c);
   if (const char* c = getenv("LM_GRAPHS")) e->use_graphs = atoi(c) != 0;
-  if (const char* c = getenv("LM_BN64_MASK")) e->bn64_mask = (unsigned)strtoul(c, nullptr, 0);
-  if (const char* c = getenv("LM_STEM_V2")) { const int v = atoi(c); e->stem_v2 = v < 0 ? 0 : (v > 3 ? 3 : v); }
-  if (const char* c = getenv("LM_UPSAMPLE_V2")) { const int v = atoi(c); e->upsample_v2 = v < 0 ? 0 : (v > 2 ? 2 : v); }
   if (const char* c = getenv("LM_CCL_RULE")) e->post.ccl_rule = atoi(c) != 0;
   if (const char* c = getenv("LM_MERGE_CTAS")) e->post.merge_ctas = atoi(c) > 0 ? atoi(c) : 0;
   if (const char* c = getenv("LM_CHUNK_KB_WIDE")) { int v = atoi(c); if (v >= 1) e->chunk_kb_wide = v; }
   RC(conv_tc_prepare());
-  RC(conv_tc_pair_prepare());
   CU(cudaStreamCreateWithFlags(&e->st, cudaStreamNonBlocking));
   for (int i = 0; i < 8; ++i) CU(cudaEventCreate(&e->ev[i]));
   for (int i = 0; i < 2; ++i) CU(cudaEventCreate(&e->ev_conv[i]));
@@ -777,7 +756,6 @@ int lm_load_weights(lm_engine* e, int slot, const float* blob, size_t n_floats, 
     p.out = L.dst >= 0 ? e->act[L.dst] : nullptr;
     p.out_pool = L.dst_pool >= 0 ? e->act[L.dst_pool] : nullptr;
     p.head_w = s.head_w; p.head_b = s.head_b; p.K = K;
-    p.tile_n = ((e->bn64_mask >> i) & 1u) ? 64 : 0;
     s.params[i] = p;
     int r = make_conv_maps(&s.maps[i], e->act[L.src0], L.src1 >= 0 ? e->act[L.src1] : nullptr, s.lw[i].w, p, e->B);
     if (r) return fail(r, "make_conv_maps failed for layer %d: %d", i, r);
@@ -1244,15 +1222,9 @@ int lm_set_option(lm_engine* e, const char* key, int value) {
   if (!e || !key) return fail(-1, "lm_set_option: NULL argument");
   e->graph_epoch++;   // captured forwards bake the kernel choices in
   if (!strcmp(key, "graphs")) { e->use_graphs = value != 0; return 0; }
-  if (!strcmp(key, "bn64_mask")) { e->bn64_mask = (unsigned)value; return 0; }   // takes effect at the next lm_load_weights
   if (!strcmp(key, "time_convs")) { e->time_convs = value != 0; e->ev_used = 0; return 0; }
   if (!strcmp(key, "post_debug_stage")) { e->post.debug_stage = value; return 0; }
   if (!strcmp(key, "chunk_kb")) { if (value < 1) return fail(-1, "chunk_kb must be >= 1"); e->chunk_kb = e->chunk_kb_wide = value; return 0; }
-  if (!strcmp(key, "dual_issue")) { e->dual_issue = value != 0; return 0; }
-  if (!strcmp(key, "cta_pairs")) { e->cta_pairs = value != 0; return 0; }
-  if (!strcmp(key, "weight_mcast")) { if (value != 0 && value != 2) return fail(-1, "weight_mcast must be 0 or 2"); e->weight_mcast = value; return 0; }
-  if (!strcmp(key, "stem_v2")) { if (value < 0 || value > 3) return fail(-1, "stem_v2 must be 0, 1, 2 or 3"); e->stem_v2 = value; return 0; }
-  if (!strcmp(key, "upsample_v2")) { e->upsample_v2 = value < 0 ? 0 : (value > 2 ? 2 : value); return 0; }
   if (!strcmp(key, "ccl_rule")) { e->post.ccl_rule = value != 0; return 0; }
   if (!strcmp(key, "shard_slab_ccl")) { e->shard_slab_ccl = value != 0; return 0; }
   if (!strcmp(key, "shard_test_slabs")) { if (value < 0 || value > kShardMaxWorld) return fail(-1, "shard_test_slabs out of range"); e->shard_test_slabs = value; return 0; }

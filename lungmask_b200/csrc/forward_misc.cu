@@ -5,8 +5,8 @@
 //                      1x1 convolution (the two commute: both are linear and the bilinear weights sum
 //                      to 1), writing the hi/lo split planes the next convolution consumes.
 //   * prep_conv_weights  OIHW fp32 -> [2][tap][Cout][Cin] hi/lo operand planes (one-time, at weight load).
-// All are HBM-bound streaming kernels: each thread produces 16 bytes of each plane (CPT = 8 fp16 / 4 tf32
-// channels) so that every warp store instruction writes fully coalesced 128-byte runs.
+// All are HBM-bound streaming kernels: each thread produces 16 bytes of each plane (CPT = 8 fp16 channels)
+// so that every warp store instruction writes fully coalesced 128-byte runs.
 #include "forward_misc.cuh"
 #include "sm100_ptx.cuh"
 
@@ -18,7 +18,6 @@ constexpr int CPT = 16 / kOpBytes;  // channels per thread
 // CPT fp32 values -> 16 bytes of the hi plane and 16 bytes of the lo plane; flags values outside the format's range
 __device__ __forceinline__ void split_store(const float* v, op_t* hi_dst, op_t* lo_dst, bool& ovf) {
   uint4 h, l;
-#if LM_OPERAND_F16
   uint32_t* ph = &h.x;
   uint32_t* pl = &l.x;
 #pragma unroll
@@ -26,20 +25,14 @@ __device__ __forceinline__ void split_store(const float* v, op_t* hi_dst, op_t* 
     split_f16x2(v[2 * e], v[2 * e + 1], ph[e], pl[e]);   // packed conversions: the roundings of split_f16, two values at a time
     ovf |= !(fabsf(v[2 * e]) <= kOpMax) | !(fabsf(v[2 * e + 1]) <= kOpMax);
   }
-#else
-  float* ph = reinterpret_cast<float*>(&h.x);
-  float* pl = reinterpret_cast<float*>(&l.x);
-#pragma unroll
-  for (int e = 0; e < 4; ++e) split_tf32(v[e], ph[e], pl[e]);
-#endif
   *reinterpret_cast<uint4*>(hi_dst) = h;
   *reinterpret_cast<uint4*>(lo_dst) = l;
 }
 
-// network input of one sample: int16 HU -> (hu + 1024) / 1624 through the table (mask.py:167-168: float64 division, then
-// the cast to fp32); float volumes arrive already normalised (preproc.cu resize_kernel<float / double>)
-__device__ __forceinline__ float stem_input(const int16_t* img, size_t idx, const float* lut) {
-  int hu = img[idx];
+// network input of one sample, from its raw value: int16 HU -> (hu + 1024) / 1624 through the table (mask.py:167-168: float64
+// division, then the cast to fp32); float volumes arrive already normalised (preproc.cu resize_kernel<float / double>)
+__device__ __forceinline__ float stem_convert(int16_t raw, const float* lut) {
+  int hu = raw;
   hu = hu > 600 ? 600 : hu;  // mask.py:167 (no-op after the clip in utils.py:45)
   const int i = hu + 1024;
   // mask.py:168.  Values below -1024 never come out of preprocess; for them (and for every other int16 value) the IEEE fp32
@@ -47,152 +40,26 @@ __device__ __forceinline__ float stem_input(const int16_t* img, size_t idx, cons
   // (tests/test_host_logic.py::test_normalisation_in_fp32_is_exact) - no double-precision division in the hot loop.
   return i >= 0 ? lut[i] : __fdiv_rn((float)i, 1624.f);
 }
-__device__ __forceinline__ float stem_input(const float* img, size_t idx, const float*) { return img[idx]; }
-// the same conversion from a sample that is already in a register (stem_kernel_v3<IT, true> fetches a tile's raw samples
-// one tile ahead)
-__device__ __forceinline__ float stem_convert(int16_t raw, const float* lut) {
-  int hu = raw;
-  hu = hu > 600 ? 600 : hu;
-  const int i = hu + 1024;
-  return i >= 0 ? lut[i] : __fdiv_rn((float)i, 1624.f);
-}
 __device__ __forceinline__ float stem_convert(float raw, const float*) { return raw; }
 
-template <typename IT>
-__global__ void __launch_bounds__(256) stem_kernel(const IT* __restrict__ in, op_t* __restrict__ out,
-                                                   const float* __restrict__ w,      // [64][9]
-                                                   const float* __restrict__ bias,   // [64]
-                                                   const float* __restrict__ scale,  // [64]
-                                                   const float* __restrict__ shift,  // [64]
-                                                   int N, int H, int W, int* __restrict__ range_flag, float out_scale) {
-  __shared__ float sw[64 * 9], sb[64], ss[64], sh[64];
-  // (hu + 1024) / 1624 for every HU value the pre-processing can produce ([-1024, 600]): float64 division, then
-  // the cast to fp32 (mask.py:168,178-182), tabulated once per block instead of nine fp64 divisions per thread
-  __shared__ float lut[1625];
-  for (int i = threadIdx.x; i < 1625; i += blockDim.x) lut[i] = __fdiv_rn((float)i, 1624.f);
-  for (int i = threadIdx.x; i < 64 * 9; i += blockDim.x) sw[i] = w[i];
-  if (threadIdx.x < 64) { sb[threadIdx.x] = bias[threadIdx.x]; ss[threadIdx.x] = scale[threadIdx.x]; sh[threadIdx.x] = shift[threadIdx.x]; }
-  __syncthreads();
-  const size_t plane = (size_t)H * W;
-  constexpr int TPP = 64 / CPT;  // threads per pixel
-  const size_t total = (size_t)N * plane * TPP;
-  bool ovf = false;
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-    const int cq = (int)(t % TPP);
-    const size_t pix = t / TPP;
-    const int n = (int)(pix / plane);
-    const int r = (int)(pix - (size_t)n * plane);
-    const int y = r / W, x = r - y * W;
-    float v[9];
-#pragma unroll
-    for (int tap = 0; tap < 9; ++tap) {
-      const int yy = y + tap / 3 - 1, xx = x + tap % 3 - 1;
-      float val = 0.f;
-      if (yy >= 0 && yy < H && xx >= 0 && xx < W) val = stem_input(in, (size_t)n * plane + (size_t)yy * W + xx, lut);
-      v[tap] = val;
-    }
-    float yv[CPT];
-#pragma unroll
-    for (int e = 0; e < CPT; ++e) {
-      const int c = cq * CPT + e;
-      float s = 0.f;
-#pragma unroll
-      for (int tap = 0; tap < 9; ++tap) s = fmaf(sw[c * 9 + tap], v[tap], s);
-      yv[e] = __fmul_rn(__fadd_rn(__fmul_rn(fmaxf(s + sb[c], 0.f), ss[c]), sh[c]), out_scale);
-    }
-    op_t* o = out + ((size_t)n * 2 * plane + r) * 64 + cq * CPT;
-    split_store(yv, o, o + plane * 64, ovf);
-  }
-  if (ovf && range_flag) *range_flag = 1;
-}
-
-// stem_kernel_v2 (opt-in, lm_set_option("stem_v2"); written without GPU time left - validate with
-// LM_TEST_EXPERIMENTAL=1 pytest -m gpu before making it the default).  Same arithmetic in the same order as stem_kernel,
-// different work assignment: ncu shows stem_kernel bound by shared-memory loads (72 weight + 9 LUT loads per thread and
-// pixel, 15 % of the HBM write rate).  Here a thread owns ONE group of CPT output channels for the whole kernel, keeps
-// that group's 9 x CPT weights and 3 x CPT epilogue constants in registers, and walks quads of 4 x-adjacent pixels with
-// an 18-sample (3 x 6) input window: 4.5 LUT loads per pixel and no weight loads.
-template <int QW, typename IT>
-__global__ void __launch_bounds__(128) stem_kernel_v2(const IT* __restrict__ in, op_t* __restrict__ out,
-                                                      const float* __restrict__ w,      // [64][9]
-                                                      const float* __restrict__ bias,   // [64]
-                                                      const float* __restrict__ scale,  // [64]
-                                                      const float* __restrict__ shift,  // [64]
-                                                      int N, int H, int W, int* __restrict__ range_flag, float out_scale) {
-  __shared__ float lut[1625];
-  for (int i = threadIdx.x; i < 1625; i += blockDim.x) lut[i] = __fdiv_rn((float)i, 1624.f);
-  constexpr int TPP = 64 / CPT;  // threads per pixel quad
-  const int cq = (int)(threadIdx.x % TPP);
-  float wr[CPT][9], br[CPT], sr[CPT], hr[CPT];
-#pragma unroll
-  for (int e = 0; e < CPT; ++e) {
-    const int c = cq * CPT + e;
-#pragma unroll
-    for (int tap = 0; tap < 9; ++tap) wr[e][tap] = __ldg(w + c * 9 + tap);
-    br[e] = __ldg(bias + c); sr[e] = __ldg(scale + c); hr[e] = __ldg(shift + c);
-  }
-  __syncthreads();
-  const size_t plane = (size_t)H * W;
-  const int quads_per_row = W / QW;
-  const size_t total_quads = (size_t)N * H * quads_per_row;
-  const size_t quad0 = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) / TPP;
-  const size_t quad_step = ((size_t)gridDim.x * blockDim.x) / TPP;
-  bool ovf = false;
-  for (size_t qd = quad0; qd < total_quads; qd += quad_step) {
-    const int qx = (int)(qd % quads_per_row);
-    const size_t rowid = qd / quads_per_row;
-    const int y = (int)(rowid % H);
-    const int n = (int)(rowid / H);
-    const int x0 = qx * QW;
-    const IT* img = in + (size_t)n * plane;
-    float win[3][QW + 2];
-#pragma unroll
-    for (int dy = 0; dy < 3; ++dy) {
-      const int yy = y + dy - 1;
-#pragma unroll
-      for (int dx = 0; dx < QW + 2; ++dx) {
-        const int xx = x0 + dx - 1;
-        float val = 0.f;
-        if (yy >= 0 && yy < H && xx >= 0 && xx < W) val = stem_input(img, (size_t)yy * W + xx, lut);
-        win[dy][dx] = val;
-      }
-    }
-#pragma unroll
-    for (int px = 0; px < QW; ++px) {
-      float yv[CPT];
-#pragma unroll
-      for (int e = 0; e < CPT; ++e) {
-        float s = 0.f;
-#pragma unroll
-        for (int tap = 0; tap < 9; ++tap) s = fmaf(wr[e][tap], win[tap / 3][px + tap % 3], s);
-        yv[e] = __fmul_rn(__fadd_rn(__fmul_rn(fmaxf(s + br[e], 0.f), sr[e]), hr[e]), out_scale);
-      }
-      const size_t r = (size_t)y * W + x0 + px;
-      op_t* o = out + ((size_t)n * 2 * plane + r) * 64 + cq * CPT;
-      split_store(yv, o, o + plane * 64, ovf);
-    }
-  }
-  if (ovf && range_flag) *range_flag = 1;
-}
-
-// stem_kernel_v3 (default since round 2).  ncu / SASS of v1 and v2: instruction-bound - every thread normalised its own
-// 3 x 6 input window (the 8 channel-group threads of a pixel quad eight times the same one, with a double-precision
-// division in the fallback path: 4700 SASS instructions per quad) and reached 1.0 - 1.4 TB/s of the 6.5 TB/s it writes at.
+// stem_kernel.  ncu / SASS of round 2's earlier versions: instruction-bound - every thread normalised its own 3 x 6 input
+// window (the 8 channel-group threads of a pixel quad eight times the same one, with a double-precision division in the
+// fallback path: 4700 SASS instructions per quad) and reached 1.0 - 1.4 TB/s of the 6.5 TB/s it writes at.
 // Here a block owns an 8-row x 32-column tile of one image: the (8+2) x (32+2) normalised samples are built ONCE in shared
 // memory (zero padding included), the 64 x 9 weights sit in shared memory too ([channel group][tap][8 channels], read as
 // LDS.128 broadcasts: 18 per quad of 4 pixels), and a thread computes 8 channels of a 4-pixel quad from 18 window loads.
-// Same arithmetic in the same order as stem_kernel (fmaf over the taps 0..8 from zero, then ReLU, BN, scale).
+// Per output: fmaf over the taps 0..8 from zero, then ReLU, BN, scale.
+// ncu's stall breakdown of a version that loaded each tile in front of its barrier is led by long-scoreboard (1.8 stalled warps
+// per issue) and barrier (0.9) stalls at two blocks per SM; here every thread fetches its (at most two) raw samples of the NEXT
+// tile into registers before it computes the current one, so the loads fly during the 2400 instructions of the compute phase
+// and the fill phase is shared-memory work only.
 constexpr int S3_TH = 8, S3_TW = 32, S3_PITCH = S3_TW + 2 + 2;   // tile rows / columns, padded row pitch of the input tile
-// kPrefetch (default since call 13): ncu's stall breakdown of the plain version is led by long-scoreboard (1.8 stalled warps per
-// issue: the tile's global loads in front of the barrier) and barrier (0.9) stalls at two blocks per SM; here every thread
-// fetches its (at most two) raw samples of the NEXT tile into registers before it computes the current one, so the loads
-// fly during the 2400 instructions of the compute phase and the fill phase is shared-memory work only.
-template <typename IT, bool kPrefetch>
-__global__ void __launch_bounds__(256) stem_kernel_v3(const IT* __restrict__ in, op_t* __restrict__ out,
-                                                      const float* __restrict__ w, const float* __restrict__ bias,
-                                                      const float* __restrict__ scale, const float* __restrict__ shift,
-                                                      int N, int H, int W, int* __restrict__ range_flag, float out_scale) {
-  static_assert(CPT == 8, "stem_kernel_v3 is written for 8 channels per thread (fp16 operand planes)");
+template <typename IT>
+__global__ void __launch_bounds__(256) stem_kernel(const IT* __restrict__ in, op_t* __restrict__ out,
+                                                   const float* __restrict__ w, const float* __restrict__ bias,
+                                                   const float* __restrict__ scale, const float* __restrict__ shift,
+                                                   int N, int H, int W, int* __restrict__ range_flag, float out_scale) {
+  static_assert(CPT == 8, "stem_kernel is written for 8 channels per thread");
   __shared__ float lut[1625];
   __shared__ __align__(16) float sw[8][9][8];                 // [channel group][tap][channel within the group]
   __shared__ __align__(16) float sc[8][3][8];                 // bias / scale / shift per channel group
@@ -226,34 +93,21 @@ __global__ void __launch_bounds__(256) stem_kernel_v3(const IT* __restrict__ in,
       raw[k] = ok[k] ? img_[(size_t)yy * W + xx] : IT(0);
     }
   };
-  if (kPrefetch && (int)blockIdx.x < N * tiles_img) fetch(blockIdx.x);
+  if ((int)blockIdx.x < N * tiles_img) fetch(blockIdx.x);
   for (int tile_id = blockIdx.x; tile_id < N * tiles_img; tile_id += gridDim.x) {
     const int n = tile_id / tiles_img, r = tile_id - n * tiles_img;
     const int y0 = (r / tiles_x) * S3_TH, x0 = (r % tiles_x) * S3_TW;
-    const IT* img = in + (size_t)n * plane;
     __syncthreads();                         // the previous tile has been consumed (and, first time, the tables are ready)
-    if constexpr (kPrefetch) {
 #pragma unroll
-      for (int k = 0; k < 2; ++k) {
-        const int i = threadIdx.x + 256 * k;
-        if (i < TILE_ELEMS) {
-          const int ty = i / (S3_TW + 2), tx = i - ty * (S3_TW + 2);
-          tile[ty][tx] = ok[k] ? stem_convert(raw[k], lut) : 0.f;   // 0: zero padding of the convolution
-        }
-      }
-    } else {
-      for (int i = threadIdx.x; i < TILE_ELEMS; i += blockDim.x) {
+    for (int k = 0; k < 2; ++k) {
+      const int i = threadIdx.x + 256 * k;
+      if (i < TILE_ELEMS) {
         const int ty = i / (S3_TW + 2), tx = i - ty * (S3_TW + 2);
-        const int yy = y0 + ty - 1, xx = x0 + tx - 1;
-        float val = 0.f;                       // zero padding of the convolution
-        if (yy >= 0 && yy < H && xx >= 0 && xx < W) val = stem_input(img, (size_t)yy * W + xx, lut);
-        tile[ty][tx] = val;
+        tile[ty][tx] = ok[k] ? stem_convert(raw[k], lut) : 0.f;   // 0: zero padding of the convolution
       }
     }
     __syncthreads();
-    if constexpr (kPrefetch) {
-      if (tile_id + (int)gridDim.x < N * tiles_img) fetch(tile_id + gridDim.x);
-    }
+    if (tile_id + (int)gridDim.x < N * tiles_img) fetch(tile_id + gridDim.x);
 #pragma unroll
     for (int half = 0; half < 2; ++half) {
       const int q = slot + 32 * half;        // quad index in the tile: row q / 8, columns 4 * (q % 8) ..
@@ -302,57 +156,13 @@ __global__ void __launch_bounds__(256) stem_kernel_v3(const IT* __restrict__ in,
   if (ovf && range_flag) *range_flag = 1;
 }
 
-// One bilinear sample with a fixed operation order (explicit fused multiply-adds: both upsample kernels round alike)
-__device__ __forceinline__ float bilerp(float p00, float p01, float p10, float p11, float lx0, float lx1, float ly0, float ly1) {
-  const float top = __fmaf_rn(lx1, p01, __fmul_rn(lx0, p00));
-  const float bot = __fmaf_rn(lx1, p11, __fmul_rn(lx0, p10));
-  return __fmaf_rn(ly1, bot, __fmul_rn(ly0, top));
-}
-
-// in: [N][h][w][C] fp32 -> out: [N][2][2h][2w][C] split planes. PyTorch semantics (align_corners=False):
-// src = max(0.5*(dst+0.5)-0.5, 0), i0 = (int)src, i1 = i0 + (i0 < size-1), l1 = src - i0, l0 = 1 - l1.
-__global__ void __launch_bounds__(256) upsample2x_kernel(const float* __restrict__ in, op_t* __restrict__ out,
-                                                         int N, int h, int w, int C, int* __restrict__ range_flag, float out_scale) {
-  const int cq_per_pix = C / CPT;
-  bool ovf = false;
-  const int H = 2 * h, W = 2 * w;
-  const size_t oplane = (size_t)H * W;
-  const size_t total = (size_t)N * oplane * cq_per_pix;
-  for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-    const int cq = (int)(t % cq_per_pix);
-    const size_t pix = t / cq_per_pix;
-    const int n = (int)(pix / oplane);
-    const int r = (int)(pix - (size_t)n * oplane);
-    const int y = r / W, x = r - y * W;
-    const float sy = fmaxf(0.5f * ((float)y + 0.5f) - 0.5f, 0.f), sx = fmaxf(0.5f * ((float)x + 0.5f) - 0.5f, 0.f);
-    const int y0 = (int)sy, x0 = (int)sx;
-    const int y1 = y0 + (y0 < h - 1 ? 1 : 0), x1 = x0 + (x0 < w - 1 ? 1 : 0);
-    const float ly1 = sy - (float)y0, ly0 = 1.f - ly1, lx1 = sx - (float)x0, lx0 = 1.f - lx1;
-    const float* base = in + (size_t)n * h * w * C + cq * CPT;
-    float vv[CPT];
-#pragma unroll
-    for (int q = 0; q < CPT / 4; ++q) {
-      const float4 p00 = __ldg(reinterpret_cast<const float4*>(base + ((size_t)y0 * w + x0) * C) + q);
-      const float4 p01 = __ldg(reinterpret_cast<const float4*>(base + ((size_t)y0 * w + x1) * C) + q);
-      const float4 p10 = __ldg(reinterpret_cast<const float4*>(base + ((size_t)y1 * w + x0) * C) + q);
-      const float4 p11 = __ldg(reinterpret_cast<const float4*>(base + ((size_t)y1 * w + x1) * C) + q);
-#define LM_BILERP(f, e) vv[4 * q + e] = __fmul_rn(bilerp(p00.f, p01.f, p10.f, p11.f, lx0, lx1, ly0, ly1), out_scale);
-      LM_BILERP(x, 0) LM_BILERP(y, 1) LM_BILERP(z, 2) LM_BILERP(w, 3)
-#undef LM_BILERP
-    }
-    op_t* o = out + ((size_t)n * 2 * oplane + r) * C + cq * CPT;
-    split_store(vv, o, o + oplane * C, ovf);
-  }
-  if (ovf && range_flag) *range_flag = 1;
-}
-
-// upsample2x_cells_kernel: the same samples from a cell-centred work assignment.  With scale 2 and align_corners=False
-// the output rows 2i+1 and 2i+2 both interpolate between input rows i and i+1 (weights 0.75/0.25 and 0.25/0.75; the
-// frame rows 0 and 2h-1 take weight 1/0 and a clamped partner), and likewise for columns: a thread owns the CELL between
-// input pixels (i, j) and (i+1, j+1), i in [-1, h-1], j in [-1, w-1], loads its four corners ONCE (CPT channels each) and
-// writes the (up to) 2 x 2 output pixels - 1 load per output instead of 4, and no 64-bit index arithmetic per output.
-// The per-row / per-column (index, weight) pairs are derived with upsample2x_kernel's own formula, so both kernels
-// produce identical bits.
+// in: [N][h][w][C] fp32 -> out: [N][2][2h][2w][C] split planes.  PyTorch semantics (align_corners=False), per output
+// row / column o: src = max(0.5*(o+0.5)-0.5, 0), i0 = (int)src, i1 = i0 + (i0 < size-1), l1 = src - i0, l0 = 1 - l1 (up_axis).
+// Cell-centred work assignment: with scale 2 the output rows 2i+1 and 2i+2 both interpolate between input rows i and i+1
+// (weights 0.75/0.25 and 0.25/0.75; the frame rows 0 and 2h-1 take weight 1/0 and a clamped partner), and likewise for
+// columns: a thread owns the CELL between input pixels (i, j) and (i+1, j+1), i in [-1, h-1], j in [-1, w-1], loads its four
+// corners ONCE (CPT channels each) and writes the (up to) 2 x 2 output pixels - 1 load per output instead of 4, and no 64-bit
+// index arithmetic per output.
 __device__ __forceinline__ void up_axis(int o, int n_in, int& i0, int& i1, float& l0, float& l1) {
   const float s = fmaxf(0.5f * ((float)o + 0.5f) - 0.5f, 0.f);
   i0 = (int)s;
@@ -360,15 +170,14 @@ __device__ __forceinline__ void up_axis(int o, int n_in, int& i0, int& i1, float
   l1 = s - (float)i0;
   l0 = 1.f - l1;
 }
-// kStatic (default): for every output row the pair (i0, i1) that up_axis() names IS the pair of rows (ya, yb) the row's cell
-// loads - frame cells included: row 0 names (0, 1), row 2h-1 names (h-1, h-1) - and likewise per column
+// For every output row the pair (i0, i1) that up_axis() names IS the pair of rows (ya, yb) the row's cell loads - frame cells
+// included: row 0 names (0, 1), row 2h-1 names (h-1, h-1) - and likewise per column
 // (tests/test_host_logic.py::test_upsample_cell_corners_are_the_rows_the_formula_names), so the corners are indexed
-// statically.  The run-time selection of the first version (kStatic = false, kept for the bit-identity test) put the 32
-// corner values into local memory (32 LDL + 8 STL per cell in the SASS) and hid from the compiler that the two samples of
-// a cell column share bilerp()'s `top` / `bot` terms: 921 -> 712 SASS instructions per cell, in an issue-bound kernel.
-template <bool kStatic>
-__global__ void __launch_bounds__(256, kStatic ? 3 : 0) upsample2x_cells_kernel(const float* __restrict__ in, op_t* __restrict__ out,
-                                                               int N, int h, int w, int C, int* __restrict__ range_flag, float out_scale) {
+// statically.  A run-time selection of the corners put the 32 corner values into local memory (32 LDL + 8 STL per cell in the
+// SASS) and hid from the compiler that the two samples of a cell column share the `top` / `bot` terms: 921 -> 712 SASS
+// instructions per cell, in an issue-bound kernel.
+__global__ void __launch_bounds__(256, 3) upsample2x_kernel(const float* __restrict__ in, op_t* __restrict__ out,
+                                                            int N, int h, int w, int C, int* __restrict__ range_flag, float out_scale) {
   const int cq_per_pix = C / CPT;
   const int cw = w + 1, ch = h + 1;
   const int H = 2 * h, W = 2 * w;
@@ -400,62 +209,36 @@ __global__ void __launch_bounds__(256, kStatic ? 3 : 0) upsample2x_cells_kernel(
       p[1][0][4 * q] = c.x; p[1][0][4 * q + 1] = c.y; p[1][0][4 * q + 2] = c.z; p[1][0][4 * q + 3] = c.w;
       p[1][1][4 * q] = e.x; p[1][1][4 * q + 1] = e.y; p[1][1][4 * q + 2] = e.z; p[1][1][4 * q + 3] = e.w;
     }
-    if constexpr (kStatic) {
-      float ly[2][2], lx[2][2];
+    float ly[2][2], lx[2][2];
 #pragma unroll
-      for (int d = 0; d < 2; ++d) {
-        int i0, i1;
-        up_axis(2 * ci + 1 + d, h, i0, i1, ly[d][0], ly[d][1]);
-        up_axis(2 * cj + 1 + d, w, i0, i1, lx[d][0], lx[d][1]);
+    for (int d = 0; d < 2; ++d) {
+      int i0, i1;
+      up_axis(2 * ci + 1 + d, h, i0, i1, ly[d][0], ly[d][1]);
+      up_axis(2 * cj + 1 + d, w, i0, i1, lx[d][0], lx[d][1]);
+    }
+    float top[2][CPT], bot[2][CPT];   // the horizontal interpolations per cell column: shared by the column's two samples
+#pragma unroll
+    for (int e = 0; e < CPT; ++e) {
+#pragma unroll
+      for (int dx = 0; dx < 2; ++dx) {
+        top[dx][e] = __fmaf_rn(lx[dx][1], p[0][1][e], __fmul_rn(lx[dx][0], p[0][0][e]));
+        bot[dx][e] = __fmaf_rn(lx[dx][1], p[1][1][e], __fmul_rn(lx[dx][0], p[1][0][e]));
       }
-      float top[2][CPT], bot[2][CPT];   // bilerp()'s first two lines per cell column: shared by the column's two samples
+    }
 #pragma unroll
-      for (int e = 0; e < CPT; ++e) {
+    for (int dy = 0; dy < 2; ++dy) {
+      const int y = 2 * ci + 1 + dy;
+      if (y < 0 || y >= H) continue;
 #pragma unroll
-        for (int dx = 0; dx < 2; ++dx) {
-          top[dx][e] = __fmaf_rn(lx[dx][1], p[0][1][e], __fmul_rn(lx[dx][0], p[0][0][e]));
-          bot[dx][e] = __fmaf_rn(lx[dx][1], p[1][1][e], __fmul_rn(lx[dx][0], p[1][0][e]));
-        }
-      }
+      for (int dx = 0; dx < 2; ++dx) {
+        const int x = 2 * cj + 1 + dx;
+        if (x < 0 || x >= W) continue;
+        float vv[CPT];
 #pragma unroll
-      for (int dy = 0; dy < 2; ++dy) {
-        const int y = 2 * ci + 1 + dy;
-        if (y < 0 || y >= H) continue;
-#pragma unroll
-        for (int dx = 0; dx < 2; ++dx) {
-          const int x = 2 * cj + 1 + dx;
-          if (x < 0 || x >= W) continue;
-          float vv[CPT];
-#pragma unroll
-          for (int e = 0; e < CPT; ++e) vv[e] = __fmul_rn(__fmaf_rn(ly[dy][1], bot[dx][e], __fmul_rn(ly[dy][0], top[dx][e])), out_scale);
-          const size_t r = (size_t)y * W + x;
-          op_t* o = out + ((size_t)n * 2 * oplane + r) * C + cq * CPT;
-          split_store(vv, o, o + oplane * C, ovf);
-        }
-      }
-    } else {
-#pragma unroll
-      for (int dy = 0; dy < 2; ++dy) {
-        const int y = 2 * ci + 1 + dy;
-        if (y < 0 || y >= H) continue;
-        int y0, y1; float ly0, ly1;
-        up_axis(y, h, y0, y1, ly0, ly1);
-        const int ry0 = (y0 == ya) ? 0 : 1, ry1 = (y1 == ya) ? 0 : 1;   // which of the two loaded rows (ya <= yb)
-#pragma unroll
-        for (int dx = 0; dx < 2; ++dx) {
-          const int x = 2 * cj + 1 + dx;
-          if (x < 0 || x >= W) continue;
-          int x0, x1; float lx0, lx1;
-          up_axis(x, w, x0, x1, lx0, lx1);
-          const int rx0 = (x0 == xa) ? 0 : 1, rx1 = (x1 == xa) ? 0 : 1;
-          float vv[CPT];
-#pragma unroll
-          for (int e = 0; e < CPT; ++e)
-            vv[e] = __fmul_rn(bilerp(p[ry0][rx0][e], p[ry0][rx1][e], p[ry1][rx0][e], p[ry1][rx1][e], lx0, lx1, ly0, ly1), out_scale);
-          const size_t r = (size_t)y * W + x;
-          op_t* o = out + ((size_t)n * 2 * oplane + r) * C + cq * CPT;
-          split_store(vv, o, o + oplane * C, ovf);
-        }
+        for (int e = 0; e < CPT; ++e) vv[e] = __fmul_rn(__fmaf_rn(ly[dy][1], bot[dx][e], __fmul_rn(ly[dy][0], top[dx][e])), out_scale);
+        const size_t r = (size_t)y * W + x;
+        op_t* o = out + ((size_t)n * 2 * oplane + r) * C + cq * CPT;
+        split_store(vv, o, o + oplane * C, ovf);
       }
     }
   }
@@ -468,13 +251,9 @@ __global__ void prep_conv_weights_kernel(const float* __restrict__ oihw, op_t* _
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const size_t tap = i % taps, ci = (i / taps) % Cin, co = i / ((size_t)taps * Cin);
     op_t hi, lo;
-#if LM_OPERAND_F16
     const float wv = __fmul_rn(oihw[i], w_scale);   // power-of-two scale chosen by the engine so that max |w| fits fp16
     split_f16(wv, hi, lo);
     if (!(fabsf(wv) <= kOpMax) && range_flag) *range_flag = 1;
-#else
-    split_tf32(__fmul_rn(oihw[i], w_scale), hi, lo);
-#endif
     const size_t o = (tap * Cout + co) * Cin + ci;
     out[o] = hi;
     out[total + o] = lo;
@@ -489,68 +268,31 @@ inline int grid_for(size_t total, int block, int num_sms) {
 
 }  // namespace
 
+// The stem kernel tiles each slice in 8 x 32 blocks (the engine's slices are 256 x 256); other shapes are rejected.
 template <typename IT>
 static int launch_stem_t(const IT* in, void* out, const float* w, const float* bias, const float* scale, const float* shift, int N,
-                         int H, int W, int* range_flag, float out_scale, int v2, int num_sms, cudaStream_t stream) {
-  constexpr int QW = 4;
-  if (v2 >= 2 && W % S3_TW == 0 && H % S3_TH == 0 && CPT == 8) {
-    const int tiles = N * (W / S3_TW) * (H / S3_TH);
-    const int cap = num_sms * 6;
-    if (v2 >= 3)
-      stem_kernel_v3<IT, true><<<tiles < cap ? tiles : cap, 256, 0, stream>>>(in, static_cast<op_t*>(out), w, bias, scale, shift, N, H, W,
-                                                                         range_flag, out_scale);
-    else
-      stem_kernel_v3<IT, false><<<tiles < cap ? tiles : cap, 256, 0, stream>>>(in, static_cast<op_t*>(out), w, bias, scale, shift, N, H, W,
-                                                                          range_flag, out_scale);
-  } else if (v2 && W % QW == 0) {
-    const size_t threads = (size_t)N * H * (W / QW) * (64 / CPT);
-    size_t blocks = (threads + 127) / 128;
-    const size_t cap = (size_t)num_sms * 8;
-    if (blocks > cap) blocks = cap;
-    if (blocks < 1) blocks = 1;
-    stem_kernel_v2<QW, IT><<<(int)blocks, 128, 0, stream>>>(in, static_cast<op_t*>(out), w, bias, scale, shift, N, H, W, range_flag, out_scale);
-  } else {
-    const size_t total = (size_t)N * H * W * (64 / CPT);
-    stem_kernel<IT><<<grid_for(total, 256, num_sms), 256, 0, stream>>>(in, static_cast<op_t*>(out), w, bias, scale, shift, N, H, W, range_flag, out_scale);
-  }
+                         int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream) {
+  if (W % S3_TW || H % S3_TH) return (int)cudaErrorInvalidValue;
+  const int tiles = N * (W / S3_TW) * (H / S3_TH);
+  const int cap = num_sms * 6;
+  stem_kernel<IT><<<tiles < cap ? tiles : cap, 256, 0, stream>>>(in, static_cast<op_t*>(out), w, bias, scale, shift, N, H, W, range_flag,
+                                                                 out_scale);
   return (int)cudaGetLastError();
 }
 
 int launch_stem(const int16_t* in, void* out, const float* w, const float* bias, const float* scale,
                 const float* shift, int N, int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream) {
-  return launch_stem_t<int16_t>(in, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, 0, num_sms, stream);
-}
-int launch_stem_v2(const int16_t* in, void* out, const float* w, const float* bias, const float* scale,
-                   const float* shift, int N, int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream) {
-  return launch_stem_t<int16_t>(in, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, 1, num_sms, stream);
-}
-int launch_stem_any(const int16_t* in, void* out, const float* w, const float* bias, const float* scale, const float* shift, int N, int H,
-                    int W, int* range_flag, float out_scale, int version, int num_sms, cudaStream_t stream) {
-  return launch_stem_t<int16_t>(in, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, version, num_sms, stream);
+  return launch_stem_t<int16_t>(in, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, num_sms, stream);
 }
 int launch_stem_f32(const float* in_norm, void* out, const float* w, const float* bias, const float* scale, const float* shift, int N,
-                    int H, int W, int* range_flag, float out_scale, int v2, int num_sms, cudaStream_t stream) {
-  return launch_stem_t<float>(in_norm, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, v2, num_sms, stream);
+                    int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream) {
+  return launch_stem_t<float>(in_norm, out, w, bias, scale, shift, N, H, W, range_flag, out_scale, num_sms, stream);
 }
 
 int launch_upsample2x(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
                       cudaStream_t stream) {
-  const size_t total = (size_t)N * 4 * h * w * (C / CPT);
+  const size_t total = (size_t)N * (h + 1) * (w + 1) * (C / CPT);
   upsample2x_kernel<<<grid_for(total, 256, num_sms), 256, 0, stream>>>(in, static_cast<op_t*>(out), N, h, w, C, range_flag, out_scale);
-  return (int)cudaGetLastError();
-}
-
-int launch_upsample2x_cells(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
-                            cudaStream_t stream) {
-  const size_t total = (size_t)N * (h + 1) * (w + 1) * (C / CPT);
-  upsample2x_cells_kernel<false><<<grid_for(total, 256, num_sms), 256, 0, stream>>>(in, static_cast<op_t*>(out), N, h, w, C, range_flag, out_scale);
-  return (int)cudaGetLastError();
-}
-
-int launch_upsample2x_cells_static(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
-                                   cudaStream_t stream) {
-  const size_t total = (size_t)N * (h + 1) * (w + 1) * (C / CPT);
-  upsample2x_cells_kernel<true><<<grid_for(total, 256, num_sms), 256, 0, stream>>>(in, static_cast<op_t*>(out), N, h, w, C, range_flag, out_scale);
   return (int)cudaGetLastError();
 }
 

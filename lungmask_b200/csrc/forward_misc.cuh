@@ -5,28 +5,17 @@
 #include "conv_tc.cuh"  // op_t: the operand format of the split planes
 
 namespace lm {
-// resized HU slices int16 [N][H][W] -> split planes [N][2][H][W][64]
+// resized HU slices int16 [N][H][W] -> split planes [N][2][H][W][64]; W must be a multiple of 32 and H of 8
 // (range_flag: device int set to 1 when a value leaves the operand format's range; may be nullptr)
 int launch_stem(const int16_t* in, void* out, const float* w, const float* bias, const float* scale,
                 const float* shift, int N, int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream);
-// same result from a different work assignment (weights in registers, 4-pixel quads); opt-in, see forward_misc.cu
-int launch_stem_v2(const int16_t* in, void* out, const float* w, const float* bias, const float* scale,
-                   const float* shift, int N, int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream);
-// version: 0 = stem_kernel, 1 = stem_kernel_v2, 2 = stem_kernel_v3 (shared input tile + shared weights; the default)
-int launch_stem_any(const int16_t* in, void* out, const float* w, const float* bias, const float* scale, const float* shift, int N, int H,
-                    int W, int* range_flag, float out_scale, int version, int num_sms, cudaStream_t stream);
 // the same convolution on an already normalised fp32 input [N][H][W] (float volumes, preproc.cuh launch_resize_float)
 int launch_stem_f32(const float* in_norm, void* out, const float* w, const float* bias, const float* scale, const float* shift, int N,
-                    int H, int W, int* range_flag, float out_scale, int v2, int num_sms, cudaStream_t stream);
+                    int H, int W, int* range_flag, float out_scale, int num_sms, cudaStream_t stream);
 // fp32 [N][h][w][C] -> split planes [N][2][2h][2w][C]
 // (all planes are stored as value * out_scale, a power of two chosen by the engine: conv_tc.cuh ConvParams)
 int launch_upsample2x(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
                       cudaStream_t stream);
-// same samples, one thread per cell between four input pixels (1 load per output instead of 4); see forward_misc.cu
-int launch_upsample2x_cells(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
-                            cudaStream_t stream);
-int launch_upsample2x_cells_static(const float* in, void* out, int N, int h, int w, int C, int* range_flag, float out_scale, int num_sms,
-                            cudaStream_t stream);
 // OIHW fp32 -> [2][taps][Cout][Cin] hi/lo operand planes
 int launch_prep_conv_weights(const float* oihw, void* out, int Cout, int Cin, int taps, int* range_flag, float w_scale,
                              cudaStream_t stream);

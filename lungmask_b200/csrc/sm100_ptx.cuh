@@ -48,19 +48,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// Non-blocking probe of a phase (mbarrier.test_wait): used to look one step ahead so that the ~100-cycle
-// latency of the barrier read overlaps with useful issue work instead of sitting on the critical path.
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}\n"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
 // Bounded wait: a pipeline bug traps (launch failure on the host) instead of hanging the GPU.
 #ifndef LM_MBAR_SPIN_LIMIT
 #define LM_MBAR_SPIN_LIMIT (1u << 24)   // try_wait suspends ~1 us per failed try: ~10-20 s before trapping
@@ -95,31 +82,12 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, 
       "l"(m), "r"(bar), "r"(c0), "r"(c1)
       : "memory");
 }
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, uint32_t bar,
-                                            int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes "
-      "[%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-      "l"(m), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* m, uint32_t bar,
                                             int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes "
       "[%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst),
       "l"(m), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-
-// the same load delivered to the same shared-memory offset of every CTA in `cta_mask` (one L2 read, fanned out on the way to
-// the SMs); each destination CTA's mbarrier at the offset of `bar` receives the complete_tx
-__device__ __forceinline__ void tma_load_4d_mcast(uint32_t dst, const CUtensorMap* m, uint32_t bar,
-                                                  int c0, int c1, int c2, int c3, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1, {%3, %4, %5, %6}], [%2], %7;" ::"r"(dst),
-      "l"(m), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(cta_mask)
       : "memory");
 }
 
@@ -146,10 +114,6 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-
 // ---------------------------------------------------------------- tcgen05
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_result, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
@@ -172,12 +136,6 @@ __device__ __forceinline__ void tc_fence_after() {
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
                    bar)
-               : "memory");
-}
-// the same arrive on the mbarrier at this offset in every CTA of `cta_mask` (weight stages shared by a cluster)
-__device__ __forceinline__ void umma_commit_mcast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(cta_mask)
                : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem], kind::tf32, fp32 accumulate. Single-thread issue.
@@ -266,107 +224,9 @@ __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// fp32 -> (tf32 hi, tf32 lo) split used by the 3xTF32 convolution: hi + lo == x to ~2^-22.
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-  uint32_t h, l;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x));
-  hi = __uint_as_float(h);
-  float r = x - hi;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(l) : "f"(r));
-  lo = __uint_as_float(l);
-}
-
 // Register reallocation between warpgroups (setmaxnreg: all four warps of a warpgroup execute it together).
 template <int N> __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
 template <int N> __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
-
-// ---------------------------------------------------------------- CTA pairs (cluster of 2, tcgen05 cta_group::2)
-// Used by conv_tc_pair.cu.  In a cluster launch a shared::cta address is also a valid shared::cluster address of the
-// executing CTA with the CTA's cluster rank in bit 24; clearing that bit addresses the same offset in rank 0.
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// Remote arrives of the pair kernel.  LM_PAIR_ARRIVE selects their memory semantics:
-//   0  .release.cluster  (round-1 version: a cluster-scope release in front of every arrive - measured at about 1000
-//                         cycles per arrive, profiles/r02_conv_role_stalls.md)
-//   1  default (.release.cta) - what the hand-shakes need: the data they order is TMEM (tcgen05.wait::ld +
-//      tcgen05.fence::before_thread_sync precede the arrive) or written by TMA (complete_tx), never generic stores
-//   2  .relaxed.cluster
-#ifndef LM_PAIR_ARRIVE
-#define LM_PAIR_ARRIVE 1
-#endif
-#if LM_PAIR_ARRIVE == 0
-#define LM_PAIR_SEM ".release.cluster"
-#elif LM_PAIR_ARRIVE == 1
-#define LM_PAIR_SEM ""
-#else
-#define LM_PAIR_SEM ".relaxed.cluster"
-#endif
-// arrive (count 1) on the mbarrier at the same shared-memory offset in the pair's leader CTA (rank 0)
-__device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
-  asm volatile("mbarrier.arrive" LM_PAIR_SEM ".shared::cluster.b64 _, [%0];" ::"r"(bar & kPeerBitMask) : "memory");
-}
-// leader's own arrive + transaction bytes of BOTH CTAs' loads (the peer's TMA completes on the leader's barrier)
-__device__ __forceinline__ void mbar_arrive_expect_tx_leader(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx" LM_PAIR_SEM ".shared::cluster.b64 _, [%0], %1;" ::"r"(bar & kPeerBitMask), "r"(bytes)
-               : "memory");
-}
-// TMA loads into this CTA's shared memory whose completion is signalled on the LEADER's mbarrier
-__device__ __forceinline__ void tma_load_4d_pair(uint32_t dst, const CUtensorMap* m, uint32_t bar,
-                                                 int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes "
-      "[%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst),
-      "l"(m), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_5d_pair(uint32_t dst, const CUtensorMap* m, uint32_t bar,
-                                                 int c0, int c1, int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes "
-      "[%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(dst),
-      "l"(m), "r"(bar & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t smem_result, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_result), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// tcgen05.commit of the pair's MMAs: arrives (count 1) on the mbarrier at this offset in every CTA of `cta_mask`
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(cta_mask)
-               : "memory");
-}
-// D[tmem of both CTAs] (+)= A[each CTA's own 128 rows] * B[N/2 rows from each CTA], kind::f16, M = 256
-template <bool ACC>
-__device__ __forceinline__ void umma_f16_pair_c(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc) {
-  if (ACC)
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.eq.u32 p, 1, 1;\n\t"
-                 "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc)
-                 : "memory");
-  else
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.eq.u32 p, 1, 0;\n\t"
-                 "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc)
-                 : "memory");
-}
-__device__ __forceinline__ void umma_f16_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 
 // fp32 -> (fp16 hi, fp16 lo * 2^11): hi + lo * 2^-11 == x to ~2^-22 (x - hi is exact in fp32; the scaled
 // residual keeps 11 significant bits even where x - hi would be an fp16 subnormal).  |x| must be <= 65504.
@@ -381,9 +241,6 @@ __device__ __forceinline__ void split_f16x2(float a, float b, uint32_t& hi, uint
   const __half2 l = __floats2half2_rn((a - hf.x) * 2048.f, (b - hf.y) * 2048.f);
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-__device__ __forceinline__ uint32_t pack_half2(__half a, __half b) {
-  return (uint32_t)__half_as_ushort(a) | ((uint32_t)__half_as_ushort(b) << 16);
 }
 
 }  // namespace lm

@@ -251,3 +251,12 @@ def test_graph_replay_matches_plain_launches(models):
             assert np.array_equal(plain, first) and np.array_equal(plain, again)
     finally:
         eng.close()
+
+
+@pytest.mark.parametrize("key", ["stem_v2", "upsample_v2", "cta_pairs", "weight_mcast", "dual_issue", "bn64_mask"])
+def test_removed_kernel_options_are_unknown_keys(engine, key):
+    """The forward has one stem, one upsample and one convolution kernel: the options that once selected alternatives are
+    rejected like any other unknown key instead of being accepted and ignored."""
+    from lungmask_b200 import _native
+    with pytest.raises(_native.NativeError, match="unknown key " + key):
+        engine.set_option(key, 0)

@@ -201,7 +201,7 @@ def test_lungmask_alias_package_resolves_to_engine_mirror():
 
 
 def test_upsample_cell_corners_are_the_rows_the_formula_names():
-    """forward_misc.cu upsample2x_cells_kernel<true> indexes the four loaded corners statically.  That is exact iff, for every
+    """forward_misc.cu upsample2x_kernel indexes the four loaded corners statically.  That is exact iff, for every
     output row y of a 2x bilinear upsample (align_corners=False, PyTorch's formula), the pair (i0, i1) the formula names
     equals the pair (ya, yb) the cell containing y loads - frame cells included (the same holds per column)."""
     f32 = np.float32

@@ -1,10 +1,9 @@
 #!/bin/bash
-# Builds the GPU probe binaries in-tree (git-ignored, but they travel with gpurun).  Run HERE before a gpurun call.
+# Builds the GPU probe binaries in-tree (git-ignored).
 set -e
 cd "$(dirname "$0")"
 F="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17"
-nvcc $F conv_probe.cu ../lungmask_b200/csrc/conv_tc.cu ../lungmask_b200/csrc/conv_tc_pair.cu -o conv_probe -lcuda
-nvcc $F -DLM_CONV_PROFILE conv_probe.cu ../lungmask_b200/csrc/conv_tc.cu ../lungmask_b200/csrc/conv_tc_pair.cu -o conv_probe_prof -lcuda
-nvcc $F pair_probe.cu -o pair_probe
+nvcc $F conv_probe.cu ../lungmask_b200/csrc/conv_tc.cu -o conv_probe -lcuda
+nvcc $F -DLM_CONV_PROFILE conv_probe.cu ../lungmask_b200/csrc/conv_tc.cu -o conv_probe_prof -lcuda
 [ -f umma_probe.cu ] && nvcc $F umma_probe.cu -o umma_probe -lcuda || true
-ls -la conv_probe pair_probe
+ls -la conv_probe conv_probe_prof

@@ -2,7 +2,7 @@
 // procedurally generated data (every element is a hash of its index, so the host can evaluate any
 // output pixel without holding the tensors), then times the 22 tensor-core layers of the U-Net at a
 // given batch. Test infrastructure only.
-//   usage: conv_probe [batch=8] [chunk_kb=4] [timing_only=0] [dual_issue=0] [cta_pairs=0] [reps=3] [bn64_mask=0] [weight_mcast=0]
+//   usage: conv_probe [batch=8] [chunk_kb=4] [timing_only=0] [reps=3]
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
@@ -13,7 +13,7 @@
 
 using namespace lm;
 #ifdef LM_CONV_PROFILE
-namespace lm { void conv_prof_reset(); void conv_prof_read(unsigned long long*); void conv_prof_reset_pair(); void conv_prof_read_pair(unsigned long long*); }
+namespace lm { void conv_prof_reset(); void conv_prof_read(unsigned long long*); }
 #endif
 
 #define CK(x)                                                                         \
@@ -34,23 +34,12 @@ __host__ __device__ inline float gen(uint32_t seed, uint64_t idx, bool ints) {
   if (ints) return (float)((int)(h % 5u) - 2);
   return ((h >> 8) * (1.0f / 16777216.0f) - 0.5f) * 2.0f;
 }
-__host__ __device__ inline float tf32_rna(float x) {
-  uint32_t u;
-  memcpy(&u, &x, 4);
-  u += 0x1000u; u &= 0xFFFFE000u;
-  memcpy(&x, &u, 4);
-  return x;
-}
 // operand-format split (conv_tc.cuh): value = hi + lo * kLoUnscale
 struct Split { op_t hi, lo; };
 __host__ __device__ inline Split split(float x) {
   Split s;
-#if LM_OPERAND_F16
   s.hi = __float2half_rn(x);
   s.lo = __float2half_rn((x - __half2float(s.hi)) * 2048.f);
-#else
-  s.hi = tf32_rna(x); s.lo = tf32_rna(x - s.hi);
-#endif
   return s;
 }
 __host__ __device__ inline double joined(const Split& s) { return (double)(float)s.hi + (double)(float)s.lo * (double)kLoUnscale; }
@@ -106,7 +95,6 @@ static float h_param(uint32_t seed, int c, int kind, bool ints) {
   return kind == 1 ? 1.0f + 0.3f * g : 0.2f * g;
 }
 
-static int g_dual = 0, g_pair = 0, g_mcast = 0, g_tile_n = 0;   // g_tile_n: forced output-channel tile of the layer being run (0 = auto)
 static double run_layer(const Layer& L, int N, int chunk_kb, int num_sms, bool check, bool ints, int reps) {
   const int Cin = L.C0 + L.C1;
   const float wscale = 1.0f / sqrtf((float)Cin * L.taps) * 1.7f;
@@ -143,20 +131,20 @@ static double run_layer(const Layer& L, int N, int chunk_kb, int num_sms, bool c
 
   ConvParams p{};
   p.N = N; p.H = L.H; p.W = L.W; p.C0 = L.C0; p.C1 = L.C1; p.Cout = L.Cout; p.taps = L.taps; p.mode = L.mode;
-  p.chunk_kb = chunk_kb; p.dual_issue = g_dual; p.weight_mcast = g_mcast; p.tile_n = g_tile_n; p.bias = b.bias; p.scale = b.scale; p.shift = b.shift; p.out = b.out; p.out_pool = b.pool;
+  p.chunk_kb = chunk_kb; p.bias = b.bias; p.scale = b.scale; p.shift = b.shift; p.out = b.out; p.out_pool = b.pool;
   p.head_w = b.hw; p.head_b = b.hb; p.K = L.K; p.labels = b.labels; p.scores = b.scores; p.range_flag = b.range_flag;
   p.in_unscale = 1.f; p.out_scale = 1.f;
   ConvMaps maps;
   int r = make_conv_maps(&maps, b.src0, b.src1, b.w, p, N);
   if (r) { printf("make_conv_maps failed %d\n", r); exit(2); }
   cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-  auto launch = [&]() { return g_pair ? launch_conv_tc_pair(maps, p, num_sms, 0) : launch_conv_tc(maps, p, num_sms, 0); };
+  auto launch = [&]() { return launch_conv_tc(maps, p, num_sms, 0); };
   r = launch();
   if (r) { printf("launch failed %d\n", r); exit(2); }
   CK(cudaDeviceSynchronize());
   float ms = 0;
 #ifdef LM_CONV_PROFILE
-  if (g_pair) conv_prof_reset_pair(); else conv_prof_reset();
+  conv_prof_reset();
 #endif
   if (reps > 0) {
     CK(cudaEventRecord(e0));
@@ -257,18 +245,14 @@ static double run_layer(const Layer& L, int N, int chunk_kb, int num_sms, bool c
 #ifdef LM_CONV_PROFILE
   if (reps > 0) {
     unsigned long long pr[16];
-    if (g_pair) {   // counters of the pair's LEADER CTA per k-block of ONE tile pair; epilogue counters come from both CTAs
-      conv_prof_read_pair(pr);
-      for (int i = 0; i < 6; ++i) pr[i] *= 2;
-      pr[9] *= 2;
-    } else conv_prof_read(pr);
-    const int BNt = g_tile_n == 64 ? 64 : conv_tile_n(L.Cout);
+    conv_prof_read(pr);
+    const int BNt = conv_tile_n(L.Cout);
     const double tiles = (double)N * (L.H / 16) * (L.W / 8) * (L.Cout / BNt) * reps;
     const double kbs = tiles * (Cin / kBK) * L.taps;
     const double ctas = std::min<double>(num_sms, tiles / reps) * reps;
     printf("PROF  %-18s per k-block cycles: kernel %.0f | producer wait aempty %.0f bempty %.0f | mma wait tempty %.0f afull %.0f bfull %.0f issue %.0f | epi wait tfull %.0f drain %.0f, tile-epilogue per tile %.0f\n",
            L.name, pr[9] / kbs * 1.0 * 1, pr[0] / kbs, pr[1] / kbs, pr[2] / kbs, pr[3] / kbs, pr[4] / kbs, pr[5] / kbs, pr[6] / kbs, pr[7] / kbs, pr[8] / tiles);
-    if (!g_pair) printf("PROF2 %-18s issuer per k-block: first two k-steps %.0f | last two k-steps %.0f | commits %.0f | barrier waits %.0f | everything else %.0f\n",
+    printf("PROF2 %-18s issuer per k-block: first two k-steps %.0f | last two k-steps %.0f | commits %.0f | barrier waits %.0f | everything else %.0f\n",
            L.name, pr[10] / kbs, pr[11] / kbs, pr[12] / kbs, (pr[2] + pr[3] + pr[4]) / kbs,
            (double)pr[5] / kbs - (double)(pr[10] + pr[11] + pr[12] + pr[2] + pr[3] + pr[4]) / kbs);
     (void)ctas;
@@ -287,14 +271,10 @@ int main(int argc, char** argv) {
   const int batch = argc > 1 ? atoi(argv[1]) : 8;
   const int chunk = argc > 2 ? atoi(argv[2]) : 4;
   const int timing_only = argc > 3 ? atoi(argv[3]) : 0;
-  g_dual = argc > 4 ? atoi(argv[4]) : 0;
-  g_pair = argc > 5 ? atoi(argv[5]) : 0;
-  const int reps = argc > 6 ? atoi(argv[6]) : 3;   // timed repetitions per network layer (0: one untimed launch per layer, for ncu)
-  const unsigned bn64_mask = argc > 7 ? (unsigned)strtoul(argv[7], nullptr, 0) : 0u;   // network layers (bit i) forced to BN = 64 tiles
-  g_mcast = argc > 8 ? atoi(argv[8]) : 0;   // 2: weight stages multicast across clusters of two CTAs
+  const int reps = argc > 4 ? atoi(argv[4]) : 3;   // timed repetitions per network layer (0: one untimed launch per layer, for ncu)
   cudaDeviceProp prop; CK(cudaGetDeviceProperties(&prop, 0));
   const int sms = prop.multiProcessorCount;
-  printf("device %s SMs %d; batch %d chunk_kb %d dual_issue %d cta_pairs %d weight_mcast %d\n", prop.name, sms, batch, chunk, g_dual, g_pair, g_mcast);
+  printf("device %s SMs %d; batch %d chunk_kb %d\n", prop.name, sms, batch, chunk);
   if (!timing_only) {
     const Layer small[] = {
         {"ints 1tile", 16, 8, kBK, 0, 64, 9, kModeReluBn, 0},
@@ -340,14 +320,7 @@ int main(int argc, char** argv) {
       {"up3.block3+head", 256, 256, 64, 0, 64, 9, kModeHead, 3},
   };
   double total_ms = 0;
-  int li = 0;
-  for (const Layer& L : net) {
-    g_tile_n = ((bn64_mask >> li) & 1u) ? 64 : 0;
-    if (g_tile_n) printf("(BN = 64 tiles) ");
-    total_ms += run_layer(L, batch, chunk, sms, !timing_only && g_tile_n != 0, false, reps);
-    ++li;
-  }
-  g_tile_n = 0;
+  for (const Layer& L : net) total_ms += run_layer(L, batch, chunk, sms, false, false, reps);
   printf("TOTAL tensor-core layers: %.3f ms for %d slices -> %.1f slices/s (conv layers only)\n", total_ms, batch,
          batch / total_ms * 1e3);
   printf("conv_probe done\n");

@@ -1,7 +1,10 @@
-"""Table of the forward's / pre-processing's small kernels from an `ncu --set full ... --page raw --csv` export
-(tools/gpu_r2_call11.sh, gpu_r2_call12.sh: the bench command itself, LM_GRAPHS=0, first launches of each kernel).
+"""Table of the forward's / pre-processing's small kernels from an `ncu --set full ... --page raw --csv` export of the bench
+command itself (LM_GRAPHS=0, first launches of each kernel):
 
-    python tools/ncu_small_table.py gpurun_out/r11_small_raw.csv profiles/r02_call11_small_kernels.md "<title>" [hbm_peak_gbs]
+    LM_GRAPHS=0 ncu --set full -k regex:'stem_kernel|upsample2x|bodymask|resize_kernel' -c 12 -f -o small \
+        python bench.py --steps 1 --warmup 0
+    ncu -i small.ncu-rep --page raw --csv > small_raw.csv
+    python tools/ncu_small_table.py small_raw.csv profiles/r02_call11_small_kernels.md "<title>" [hbm_peak_gbs]
 """
 import csv
 import sys

@@ -1,7 +1,9 @@
-"""Per-layer table of one full 37-slice wave of the convolution kernel from an `ncu --set full ... --page raw --csv` export
-(tools/gpu_r2_call3.sh: `conv_probe 37 2 1 0 0 0` = one launch per layer in network order).
+"""Per-layer table of one full 37-slice wave of the convolution kernel from an `ncu --set full ... --page raw --csv` export of
+`tools/conv_probe 37 2 1 0` (reps = 0: one launch per layer in network order):
 
-    python tools/ncu_wave_table.py gpurun_out/r3_conv_wave_raw.csv profiles/r02_conv_wave_table.md profiles/r02_conv_traffic.json
+    ncu --set full -k regex:conv_tc_kernel -c 21 -f -o wave tools/conv_probe 37 2 1 0
+    ncu -i wave.ncu-rep --page raw --csv > wave_raw.csv
+    python tools/ncu_wave_table.py wave_raw.csv profiles/r02_conv_wave_table.md profiles/r02_conv_traffic.json
 """
 import csv
 import json
